@@ -3,6 +3,7 @@
 
   python bench.py [--config C] --gpus N --steps K --warmup W     (torchrun launches N ranks for N > 1)
   python bench.py --impl reference [--config C] ...              the reference's own CPU path on the host cores
+  python bench.py ... --dump-outputs DIR                         also write the last timed step's outputs as .npy
 
 --config (default 2 = the headline, BASELINE.json configs[1]; the other four are the parity-test shapes, measured
 to the same contract):
@@ -166,6 +167,37 @@ def xform_mag(center, scale):
     return (np.abs(np.asarray(center, np.float64)) + 100.0 * np.abs(np.asarray(scale, np.float64)))[:, None, :]
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(outputs, batch, directory, limit=DUMP_LIMIT_BYTES):
+    """Write every output as DIR/<name>.npy so that two builds can be compared array for array.  Floating-point
+    arrays keep f32/f64; integer ones are written as f64 (exact below 2^53).  When the arrays exceed `limit` bytes
+    in all, every per-sample array ([batch, ...]) keeps the same seeded sample of rows, whose row numbers go to
+    sample_rows.npy; the aggregates (loss, sums, counters) are written whole."""
+    import numpy as np
+    arrays = {}
+    for name, t in outputs.items():
+        a = t.detach().cpu().numpy()
+        arrays[name] = a if a.dtype in (np.float32, np.float64) else a.astype(np.float64)
+    per_sample = [n for n, a in arrays.items() if a.ndim >= 2 and a.shape[0] == batch]
+    header = 128                                     # bytes of an .npy header
+    total = sum(a.nbytes + header for a in arrays.values())
+    if total > limit:
+        row_bytes = sum(arrays[n].nbytes for n in per_sample) // batch
+        keep = min(batch, (limit - header - (total - row_bytes * batch)) // (row_bytes + 8))
+        if not per_sample or keep < 1:
+            raise ValueError(f"the outputs take {total} bytes and the arrays that are not per sample alone exceed "
+                             f"the {limit}-byte dump limit: nothing can be sampled")
+        rows = np.sort(np.random.default_rng(0).choice(batch, keep, replace=False))
+        for n in per_sample:
+            arrays[n] = arrays[n][rows]
+        arrays["sample_rows"] = rows.astype(np.float64)
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, name + ".npy"), a)
+
+
 # =========================================================================================================
 # Workloads
 # =========================================================================================================
@@ -197,6 +229,10 @@ class Workload:
 
     def begin_epoch(self):
         pass
+
+    def outputs(self, steps):
+        """name -> device tensor: what a caller of the timed path holds after the last of `steps` timed steps."""
+        raise NotImplementedError
 
     launches_per_step = 1
 
@@ -402,6 +438,12 @@ class FusedWorkload(Workload):
         if self.epoch_loss is not None:
             return float(self.epoch_loss.item()) / (self.world * steps)
         return float(self.bound[(steps - 1) % self.R].loss.item())
+
+    def outputs(self, steps):
+        b = self.bound[(steps - 1) % self.R]
+        # at N > 1 without --global-loss, b.loss is the shared accumulator: the epoch's loss sum over all ranks
+        return {"preds": b.preds, "hm_preds": b.hm_preds, "idx": b.idx, "target_weight": b.weight,
+                "loss_sums": b.sums, "loss" if self.epoch_loss is None else "epoch_loss_sum": b.loss}
 
 
 class DecodeWorkload(Workload):
@@ -632,6 +674,13 @@ class DecodeWorkload(Workload):
     def loss_check(self, steps):
         return None
 
+    def outputs(self, steps):
+        b = self.bound[(steps - 1) % self.R]
+        out = {"preds": b.preds, "hm_preds": b.hm_preds, "idx": b.idx}
+        if self.metrics:
+            out["counters"] = self.total            # running PCK/AUC/EPE counters over the timed steps
+        return out
+
 
 class SimdrWorkload(Workload):
     """Config 3: keypoints_from_simdr on 2 x [4096, 21, 512] f32."""
@@ -704,6 +753,10 @@ class SimdrWorkload(Workload):
 
     def loss_check(self, steps):
         return None
+
+    def outputs(self, steps):
+        b = self.bound[(steps - 1) % self.R]
+        return {"preds": b.out, "idx": b.idx}
 
 
 def make_workload(args, rank, world, dev):
@@ -936,6 +989,8 @@ def run_gpu_arm(args, rank, local_rank, world):
     clocks = sampler.stop()
     ms_total = e0.elapsed_time(e1)
     loss_val = wl.loss_check(args.steps)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(wl.outputs(args.steps), wl.B, args.dump_outputs)
 
     # ---- parity of the measured outputs (rank 0; before anything else touches the output buffers) -----------
     parity = None
@@ -1067,6 +1122,10 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-parity", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write rank 0's outputs of the last step as DIR/<name>.npy (f32/f64, "
+                         "at most 64 MB in all); configs 2/5 at N > 1 without --global-loss write the epoch's loss sum "
+                         "over all ranks as epoch_loss_sum instead of the step's loss")
     # accepted for old command lines (all are the default behaviour now)
     ap.add_argument("--no-graph", action="store_true", help=argparse.SUPPRESS)
     ap.add_argument("--no-graph-all", action="store_true", help=argparse.SUPPRESS)

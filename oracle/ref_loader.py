@@ -1,11 +1,11 @@
 """Loader for the UNMODIFIED reference hot-path modules (test infrastructure only).
 
 This file is part of ``oracle/`` — the checker, never the product.  It imports the
-reference's own Python files from ``/root/reference`` *by file path* so that
+reference's own Python files (``REF_ROOT``) *by file path* so that
 
   * ``oracle/make_golden.py`` can generate the golden vectors in ``tests/golden/`` and
   * ``tests/test_oracle_vs_reference.py`` can pin the numpy restatement (``oracle/np_oracle.py``)
-    against the executed reference (skipped when ``/root/reference`` is absent, e.g. on the GPU box).
+    against the executed reference (skipped when the reference tree is absent).
 
 Nothing under ``litehandnet_b200/`` imports this module.
 
@@ -20,7 +20,8 @@ import os
 import sys
 import types
 
-REF_ROOT = os.environ.get("LHN_REFERENCE_ROOT", "/root/reference")
+# the original project's source tree: LHN_REFERENCE_ROOT, else the copy oracle/build_ref.py stages in oracle/_ref
+REF_ROOT = os.environ.get("LHN_REFERENCE_ROOT", os.path.join(os.path.dirname(os.path.abspath(__file__)), "_ref"))
 
 _LOADED = {}
 

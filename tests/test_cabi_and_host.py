@@ -225,6 +225,40 @@ def test_bench_reference_arm_prints_contract_line():
     assert line["impl"] == "reference" and line["value"] > 0 and line["cpu_baseline"]["kind"] in ("reference", "port")
 
 
+def test_bench_dump_outputs_types_and_sampling(tmp_path):
+    """bench.dump_outputs: floats keep their precision, integers become exact f64; over the size limit every
+    per-sample array keeps the same seeded rows (listed in sample_rows.npy) and the aggregates stay whole."""
+    import bench
+    B = 1000
+    out = {"preds": torch.arange(B * 6, dtype=torch.float32).reshape(B, 2, 3),
+           "idx": torch.arange(B * 2, dtype=torch.int32).reshape(B, 2),
+           "loss_sums": torch.tensor([1.0, 2.0, 3.0, 4.0], dtype=torch.float64),
+           "counters": torch.arange(B, dtype=torch.int64)}
+
+    def load(d):
+        return {f[:-4]: np.load(d / f) for f in os.listdir(d)}
+
+    bench.dump_outputs(out, B, str(tmp_path / "whole"))
+    whole = load(tmp_path / "whole")
+    assert sorted(whole) == sorted(out)
+    assert whole["preds"].dtype == np.float32 and whole["idx"].dtype == np.float64 and whole["counters"].dtype == np.float64
+    for n, t in out.items():
+        assert np.array_equal(whole[n], t.numpy()), n
+    limit = 24000
+    bench.dump_outputs(out, B, str(tmp_path / "a"), limit=limit)
+    bench.dump_outputs(out, B, str(tmp_path / "b"), limit=limit)
+    a, b = load(tmp_path / "a"), load(tmp_path / "b")
+    assert sorted(a) == sorted(sorted(out) + ["sample_rows"]) and sorted(b) == sorted(a)
+    assert all(np.array_equal(a[n], b[n]) for n in a), "the sample must not change from run to run"
+    assert sum(os.path.getsize(tmp_path / "a" / f"{n}.npy") for n in a) <= limit
+    rows = a["sample_rows"].astype(np.int64)
+    assert 0 < len(rows) < B and np.all(np.diff(rows) > 0)
+    assert np.array_equal(a["preds"], whole["preds"][rows]) and np.array_equal(a["idx"], whole["idx"][rows])
+    assert np.array_equal(a["counters"], whole["counters"]) and np.array_equal(a["loss_sums"], whole["loss_sums"])
+    with pytest.raises(ValueError):                  # aggregates alone over the limit: nothing to sample
+        bench.dump_outputs({"counters": out["counters"]}, B, str(tmp_path / "c"), limit=4000)
+
+
 def test_decode_params_cache_is_keyed_on_every_field(lib_path):
     """ops._decode_params shares one read-only struct between calls with equal arguments (host time per launch);
     any differing field — flags included — must give a different struct."""

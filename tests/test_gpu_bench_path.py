@@ -8,6 +8,10 @@ exactly as bench.py does and compare every step with the reference's CPU pipelin
 keypoints_from_heatmaps('unbiased'); top_down_eval.py:375-463, loss/heatmapLoss.py:242-265) on ALL 1024
 samples: argmax indices bit-exact, coordinates 1e-5 element-wise, loss 1e-5 relative.
 """
+import os
+import subprocess
+import sys
+
 import numpy as np
 import pytest
 import torch
@@ -260,3 +264,41 @@ def test_ops_follow_the_tensors_device():
     assert np.array_equal(out["idx"].cpu().numpy(), ref[1])
     with pytest.raises(L.LhnError):
         ops.decode_heatmap(s[0], L.MASK_NEG1, L.REFINE_NONE, L.XFORM_CENTER_SCALE, s[4].to("cuda:0"), s[5])
+
+
+def test_bench_dump_outputs_are_the_last_timed_step(tmp_path):
+    """bench.py --dump-outputs: the same arguments give the same arrays, and --steps decides which rotating input set
+    the last timed step decoded (config 1 with three sets: steps 1 and 4 end on set 0, steps 5 on set 1).  The run
+    exits non-zero when its outputs fail the oracle parity check."""
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+
+    def run(steps):
+        d = tmp_path / f"steps{steps}"
+        r = subprocess.run([sys.executable, "bench.py", "--config", "1", "--rotate", "3", "--steps", str(steps), "--warmup", "3",
+                            "--no-e2e", "--no-cpu-baseline", "--dump-outputs", str(d)],
+                           cwd=root, capture_output=True, text=True, timeout=600)
+        assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-3000:]
+        return {f[:-4]: np.load(d / f) for f in os.listdir(d)}
+
+    one, four, five = run(1), run(4), run(5)
+    assert sorted(one) == ["hm_preds", "idx", "preds"]
+    assert one["preds"].shape == (64, 21, 3) and one["preds"].dtype == np.float32 and one["idx"].dtype == np.float64
+    assert all(np.array_equal(one[n], four[n], equal_nan=True) for n in one)
+    assert not np.array_equal(four["idx"], five["idx"])
+
+
+@pytest.mark.parametrize("config,names", [
+    (2, {"preds": (64, 21, 3), "hm_preds": (64, 21, 3), "idx": (64, 21), "target_weight": (64, 21), "loss_sums": (4,),
+         "loss": (1,)}),
+    (3, {"preds": (64, 21, 3), "idx": (64, 21, 2)}),
+    (4, {"preds": (64, 16, 3), "hm_preds": (64, 16, 3), "idx": (64, 16), "counters": (25 * 16,)})])
+def test_bench_dump_outputs_of_every_workload(tmp_path, config, names):
+    """bench.py --dump-outputs writes each workload's outputs under their names, in f32 or f64."""
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    r = subprocess.run([sys.executable, "bench.py", "--config", str(config), "--batch", "64", "--steps", "3", "--warmup", "3",
+                        "--no-e2e", "--no-cpu-baseline", "--dump-outputs", str(tmp_path)],
+                       cwd=root, capture_output=True, text=True, timeout=600)
+    assert r.returncode == 0, r.stdout[-2000:] + r.stderr[-3000:]
+    got = {f[:-4]: np.load(tmp_path / f) for f in os.listdir(tmp_path)}
+    assert {n: a.shape for n, a in got.items()} == names
+    assert all(a.dtype in (np.float32, np.float64) for a in got.values())

@@ -1,6 +1,6 @@
-"""CPU, only where /root/reference is mounted (this container): the numpy oracle against the EXECUTED,
-unmodified reference on fresh seeds (the committed golden vectors cover the GPU box, where the reference
-does not exist — tests/test_oracle_golden.py).  Skipped when the reference tree is absent."""
+"""CPU, only where the original project's source tree is present (LHN_REFERENCE_ROOT, or the copy staged in
+oracle/_ref): the numpy oracle against the EXECUTED, unmodified reference on fresh seeds.  Skipped without it;
+tests/test_oracle_golden.py checks the oracle against the reference's stored outputs everywhere."""
 import numpy as np
 import pytest
 import torch
@@ -10,7 +10,8 @@ from oracle import ref_loader
 from litehandnet_b200 import synth
 from conftest import assert_coords_close
 
-pytestmark = pytest.mark.skipif(not ref_loader.available(), reason="reference tree not mounted")
+pytestmark = pytest.mark.skipif(not ref_loader.available(),
+                                reason="the original project's sources are not present (set LHN_REFERENCE_ROOT)")
 
 
 @pytest.fixture(scope="module")

@@ -295,6 +295,35 @@ LHN_API int lhn_render_loss_backward(const void* hm, int dtype, int64_t B, int K
                                      int vis_stride, const double* sums, int sum_reduction, float scale,
                                      const float* grad_out, void* grad, lhn_stream_t stream);
 
+/* The fused loss AND its gradient in one pass over hm (one read, one write): the same inputs as
+ * lhn_render_loss_backward, plus what lhn_fused_render_loss_decode reports for the loss — out_weight
+ * [B*S*K] (optional), sums f64 [4] = (S_pos, S_neg, N_pos, numel) (optional), loss f32 [1] (optional,
+ * as lhn_loss_finalize with sum_reduction and loss_scale).  N_pos is counted from the joints before the
+ * first gradient element is written, so it equals the fused forward's.  grad (contiguous [B, S*K, H, W],
+ * heatmap dtype) is d loss / d hm for an upstream gradient grad_scale[0] (f32 [1] device pointer, NULL = 1):
+ * coefficient (float)(c * loss_scale * grad_scale[0]) — bit-identical to lhn_render_loss_backward run
+ * with grad_out = grad_scale on these sums.  used_scale (f32 [1], optional) receives the value assumed.
+ * workspace: lhn_render_loss_grad_workspace_bytes(B, K, num_stacks) bytes, 16-byte aligned, zero before
+ * the first call and left zero.  One cooperative launch (a grid-wide barrier after the count). */
+LHN_API int64_t lhn_render_loss_grad_workspace_bytes(int64_t B, int K, int num_stacks);
+LHN_API int lhn_render_loss_grad(const void* hm, int dtype, int64_t B, int K, int H, int W,
+                                 int64_t stride_b, int64_t stride_c, const lhn_render_params* rp,
+                                 const float* joints, int joints_stride, const float* vis, int vis_stride,
+                                 float* out_weight, void* workspace, int64_t workspace_bytes, double* sums,
+                                 int sum_reduction, float loss_scale, float* loss, const float* grad_scale,
+                                 float* used_scale, void* grad, lhn_stream_t stream);
+
+/* The backward of lhn_render_loss_grad: if grad_out[0] (NULL = 1) is bitwise equal to used_scale[0], the
+ * gradient already in `grad` is the answer and nothing is written; otherwise grad is overwritten exactly
+ * as lhn_render_loss_backward(grad_out) would.  recomputed (int32 [1], optional) receives 0 or 1.  One
+ * launch of about one wave either way. */
+LHN_API int lhn_render_loss_backward_cond(const void* hm, int dtype, int64_t B, int K, int H, int W,
+                                          int64_t stride_b, int64_t stride_c, const lhn_render_params* rp,
+                                          const float* joints, int joints_stride, const float* vis,
+                                          int vis_stride, const double* sums, int sum_reduction, float scale,
+                                          const float* grad_out, const float* used_scale, int32_t* recomputed,
+                                          void* grad, lhn_stream_t stream);
+
 /* KLDiscretLoss backward (centernet_simdr_loss.py:27-39): grad_x[b,j,i] = grad_out * scale *
  * SmoothL1'(out_x - tgt_x) * mean_b(weight[b,j]) / (K * B * Lx), likewise grad_y.  workspace:
  * lhn_simdr_backward_workspace_bytes(K) bytes. */

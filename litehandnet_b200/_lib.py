@@ -41,6 +41,7 @@ EXPORTS = [
     "lhn_evaluate_pck", "lhn_flip_back", "lhn_fused_workspace_bytes", "lhn_fused_render_loss_decode",
     "lhn_fused_render_loss_decode_xch", "lhn_decode_heatmap_pck_xch", "lhn_exchange_flush",
     "lhn_loss_backward", "lhn_render_loss_backward", "lhn_simdr_backward_workspace_bytes",
+    "lhn_render_loss_grad_workspace_bytes", "lhn_render_loss_grad", "lhn_render_loss_backward_cond",
     "lhn_simdr_smoothl1_backward", "lhn_mpii_pckh_accumulate", "lhn_region_bbox_decode", "lhn_heatmap_nms",
     "lhn_vector_nms", "lhn_refine_points", "lhn_decode_heatmap_roi", "lhn_box_nms", "lhn_render_region_wh", "lhn_dark_refine_points",
 ]
@@ -104,6 +105,12 @@ def _declare(lib):
     lib.lhn_loss_backward.argtypes = [vp, vp, vp, i32, i64, i64, i32, f32, vp, i32, f32, vp, vp, vp]
     lib.lhn_render_loss_backward.argtypes = [vp, i32, i64, i32, i32, i32, i64, i64, C.POINTER(RenderParams),
                                              vp, i32, vp, i32, vp, i32, f32, vp, vp, vp]
+    lib.lhn_render_loss_grad_workspace_bytes.argtypes = [i64, i32, i32]
+    lib.lhn_render_loss_grad_workspace_bytes.restype = i64
+    lib.lhn_render_loss_grad.argtypes = [vp, i32, i64, i32, i32, i32, i64, i64, C.POINTER(RenderParams),
+                                         vp, i32, vp, i32, vp, vp, i64, vp, i32, f32, vp, vp, vp, vp, vp]
+    lib.lhn_render_loss_backward_cond.argtypes = [vp, i32, i64, i32, i32, i32, i64, i64, C.POINTER(RenderParams),
+                                                  vp, i32, vp, i32, vp, i32, f32, vp, vp, vp, vp, vp]
     lib.lhn_simdr_backward_workspace_bytes.argtypes = [i32]
     lib.lhn_simdr_backward_workspace_bytes.restype = i64
     lib.lhn_simdr_smoothl1_backward.argtypes = [vp, vp, vp, vp, vp, i32, i64, i32, i32, i32, f32, vp, vp, i64,

@@ -17,7 +17,7 @@ LIBDIR = os.path.join(HERE, "lib")
 OBJDIR = os.path.join(LIBDIR, "obj")
 LIB = os.path.join(LIBDIR, "liblhn.so")
 SOURCES = ["lhn_heatmap.cu", "lhn_heatmap_team_launch.cu", "lhn_heatmap_team_f32.cu", "lhn_heatmap_team_bf16.cu",
-           "lhn_heatmap_team_f16.cu", "lhn_loss_render.cu", "lhn_loss_multi.cu", "lhn_backward.cu", "lhn_simdr.cu", "lhn_simdr_heads.cu", "lhn_metrics.cu", "lhn_exchange.cu", "lhn_region.cu", "lhn_host.cu"]
+           "lhn_heatmap_team_f16.cu", "lhn_loss_render.cu", "lhn_loss_multi.cu", "lhn_backward.cu", "lhn_loss_grad.cu", "lhn_simdr.cu", "lhn_simdr_heads.cu", "lhn_metrics.cu", "lhn_exchange.cu", "lhn_region.cu", "lhn_host.cu"]
 HEADERS = [os.path.join(CSRC, "lhn_common.cuh"), os.path.join(CSRC, "lhn_exchange.cuh"), os.path.join(CSRC, "lhn_heatmap.cuh"), os.path.join(CSRC, "lhn_heatmap_team.cuh"), os.path.join(HERE, "..", "include", "lhn.h")]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC,-fvisibility=hidden", "--expt-relaxed-constexpr"]

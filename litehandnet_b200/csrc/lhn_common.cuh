@@ -204,6 +204,47 @@ __device__ __forceinline__ float exp_f32_from_f64(double a) {
 }
 
 // ---------------------------------------------------------------------------------------------
+// gradient stores and loss coefficients, shared by lhn_backward.cu and lhn_loss_grad.cu so that the
+// two-pass and the one-pass backward write bit-identical gradients
+// ---------------------------------------------------------------------------------------------
+template <typename T> struct Store4;
+template <> struct Store4<float> {
+  static __device__ __forceinline__ void st(float* p, float4 v) { *reinterpret_cast<float4*>(p) = v; }
+  static __device__ __forceinline__ float from(float v) { return v; }
+};
+template <> struct Store4<__nv_bfloat16> {
+  static __device__ __forceinline__ void st(__nv_bfloat16* p, float4 v) {
+    __nv_bfloat162 a = __floats2bfloat162_rn(v.x, v.y), b = __floats2bfloat162_rn(v.z, v.w);
+    uint2 r;
+    r.x = *reinterpret_cast<uint32_t*>(&a); r.y = *reinterpret_cast<uint32_t*>(&b);
+    *reinterpret_cast<uint2*>(p) = r;
+  }
+  static __device__ __forceinline__ __nv_bfloat16 from(float v) { return __float2bfloat16_rn(v); }
+};
+template <> struct Store4<__half> {
+  static __device__ __forceinline__ void st(__half* p, float4 v) {
+    __half2 a = __floats2half2_rn(v.x, v.y), b = __floats2half2_rn(v.z, v.w);
+    uint2 r;
+    r.x = *reinterpret_cast<uint32_t*>(&a); r.y = *reinterpret_cast<uint32_t*>(&b);
+    *reinterpret_cast<uint2*>(p) = r;
+  }
+  static __device__ __forceinline__ __half from(float v) { return __float2half_rn(v); }
+};
+
+// coefficients of the positive / negative elements from the forward sums (f64 -> f32 once)
+__device__ __forceinline__ void loss_coefs(const double* sums, int loss_mode, int sum_reduction, float scale,
+                                           const float* grad_out, float& cpos, float& cneg) {
+  const double npos = sums[2], numel = sums[3];
+  double cp, cn;
+  if (loss_mode == LHN_LOSS_DISTANCE_BALANCE) { cp = 2.0 * 0.1 / (npos + 1.0); cn = 2.0 / (numel - npos + 1.0); }
+  else if (loss_mode == LHN_LOSS_JOINTS_MSE) { cp = cn = 1.0 / numel; }
+  else { cp = cn = 2.0 / numel; }
+  if (sum_reduction) { cp *= numel; cn *= numel; }
+  const double g = (double)scale * (grad_out ? (double)grad_out[0] : 1.0);
+  cpos = (float)(cp * g); cneg = (float)(cn * g);
+}
+
+// ---------------------------------------------------------------------------------------------
 // mbarrier + TMA bulk copy (cp.async.bulk, 1-D: no tensor map needed for contiguous planes)
 // ---------------------------------------------------------------------------------------------
 __device__ __forceinline__ uint32_t smem_u32(const void* p) {

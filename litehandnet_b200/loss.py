@@ -89,6 +89,38 @@ class _FusedHeatmapLossFn(torch.autograd.Function):
         return ops.render_loss_backward(output, joints, vis, render, sums, reduction, 1.0, grad_out), None, None, None, None
 
 
+class _FusedHeatmapLossOnePassFn(torch.autograd.Function):
+    """The fused entry with the gradient written in the forward (lhn_render_loss_grad: one read of the output,
+    one write of the gradient).  The gradient assumes the upstream value ``expected``; the backward
+    (lhn_render_loss_backward_cond) returns it as is when autograd delivers exactly that value, and rewrites it
+    as the two-pass backward would otherwise.  The gradient buffer is allocated here, in the forward."""
+
+    @staticmethod
+    def forward(ctx, output, joints, vis, render, reduction, expected):
+        r = ops.render_loss_grad(output.detach(), joints, vis, render, reduction, 1.0, expected)
+        ctx.save_for_backward(output.detach(), joints, vis, r["sums"], r["used_scale"])
+        # the gradient is an intermediate, kept on ctx and released in backward: handed back with no other
+        # reference, autograd adopts it as output.grad instead of copying it
+        ctx.grad = r["grad"]
+        ctx.cfg = (render, reduction)
+        ctx.mark_non_differentiable(r["weight"])
+        return r["loss"][0], r["weight"]
+
+    @staticmethod
+    def backward(ctx, grad_out, _grad_w):
+        output, joints, vis, sums, used = ctx.saved_tensors
+        grad, ctx.grad = ctx.grad, None
+        render, reduction = ctx.cfg
+        g = ops.render_loss_backward_cond(output, joints, vis, render, sums, grad, used, reduction, 1.0, grad_out,
+                                          recomputed=_ONE_PASS_PROBE.get("recomputed"))
+        del grad
+        return g, None, None, None, None, None
+
+
+# tests: an int32 [1] CUDA tensor under "recomputed" receives which branch the conditional backward took
+_ONE_PASS_PROBE = {}
+
+
 class _SimDRLossFn(torch.autograd.Function):
     @staticmethod
     def forward(ctx, out_x, out_y, tgt_x, tgt_y, weight):
@@ -169,14 +201,26 @@ class DistanceLoss(nn.Module):
         return _HeatmapLossFn.apply(output, target, target_weight, self._mode, self.value, self.reduction)
 
     def forward_fused(self, output, joints_3d, joints_3d_visible, image_size, sigma=2,
-                      unbiased_encoding=True):
+                      unbiased_encoding=True, one_pass=False, expected_grad_out=1.0):
         """Additive fused entry (SURVEY §8b): render the target in-kernel from the joints instead of
-        reading a target tensor.  Returns (loss, target_weight [.., 1])."""
+        reading a target tensor.  Returns (loss, target_weight [.., 1]).
+
+        one_pass=True (when a gradient is needed): the loss and d loss / d output come from ONE pass over the
+        output, and ``loss.backward()`` returns that gradient without reading the output again — provided the
+        upstream gradient of the loss is bitwise ``expected_grad_out`` (a float, or a 0-dim CUDA tensor such as
+        a gradient scaler's scale times the loss weight).  Any other upstream value is still correct: the
+        backward then recomputes the gradient as the default route does.  The gradient buffer (one tensor
+        like ``output``) is allocated in the forward rather than in the backward."""
         L.require_cuda(output, "output")
         render = dict(loss_mode=self._mode, image_size=image_size, sigma=sigma, unbiased=unbiased_encoding,
                       pos_value=self.value)
-        loss, weight = _FusedHeatmapLossFn.apply(output, _as_cuda(joints_3d, output.device),
-                                                 _as_cuda(joints_3d_visible, output.device), render, self.reduction)
+        joints = _as_cuda(joints_3d, output.device)
+        vis = _as_cuda(joints_3d_visible, output.device)
+        if one_pass and torch.is_grad_enabled() and output.requires_grad:
+            loss, weight = _FusedHeatmapLossOnePassFn.apply(output, joints, vis, render, self.reduction,
+                                                            expected_grad_out)
+        else:
+            loss, weight = _FusedHeatmapLossFn.apply(output, joints, vis, render, self.reduction)
         return loss, weight.unsqueeze(-1)
 
 
@@ -281,6 +325,8 @@ class TopdownHeatmapLoss(nn.Module):
         self._image_size = cfg.DATASET.get('image_size', None)
         self._sigma = cfg.PIPELINE.get('sigma', 2)
         self._unbiased = cfg.PIPELINE.get('unbiased_encoding', True)
+        # fused entry: loss and gradient in one pass over the output (DistanceLoss.forward_fused(one_pass=True))
+        self.one_pass_grad = bool(cfg.LOSS.get('one_pass_grad', False))
 
     def forward(self, output, meta):
         loss_dict = {}
@@ -296,9 +342,10 @@ class TopdownHeatmapLoss(nn.Module):
             if meta.get('use_different_joint_weights', False) or (hasattr(ann, 'get') and ann.get('use_different_joint_weights', False)):
                 raise NotImplementedError("use_different_joint_weights: render the targets with TopDownGenerateTarget "
                                           "and pass meta['target'] / meta['target_weight'] instead of the fused entry")
+            # autograd delivers loss_weight[0] (as f32) to the heatmap term of `loss` below
             hl, target_weight = self.heatmap_loss.forward_fused(
                 output, meta['joints_3d'], meta['joints_3d_visible'], self._image_size, self._sigma,
-                self._unbiased)
+                self._unbiased, one_pass=self.one_pass_grad, expected_grad_out=float(self.loss_weight[0]))
         loss_dict['heatmap'] = self.loss_weight[0] * hl
         if self.simdr_loss is not None:
             simdr_x = meta['simdr_x'].to(device)

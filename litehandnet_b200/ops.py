@@ -477,6 +477,96 @@ def render_loss_backward(hm, joints, vis, render, sums, reduction="mean", scale=
     return grad
 
 
+_GRAD_WS = {}
+_SCALES = {}
+
+
+def render_loss_grad_workspace(device, B, K, S=1):
+    """Zeroed once per (device, stream, size); lhn_render_loss_grad leaves it zeroed."""
+    need = int(L.lib().lhn_render_loss_grad_workspace_bytes(int(B), int(K), int(S)))
+    key = (str(device), torch.cuda.current_stream(device).cuda_stream)
+    ws = _GRAD_WS.get(key)
+    if ws is None or ws.numel() < need:
+        ws = _GRAD_WS[key] = torch.zeros(need, dtype=torch.uint8, device=device)
+    return ws
+
+
+def _scale_tensor(v, device):
+    """A float or a one-element CUDA tensor -> (keep-alive f32 [1] tensor on `device`, pointer)."""
+    if isinstance(v, torch.Tensor):
+        t = L.require_cuda(v, "grad_scale").detach().to(torch.float32).reshape(1).contiguous()
+        return t, L.ptr(t)
+    key = (str(device), float(v))
+    t = _SCALES.get(key)
+    if t is None:                                  # a constant: filled once, the library only reads it
+        if len(_SCALES) > 64:
+            _SCALES.clear()
+        t = _SCALES[key] = torch.full((1,), float(v), dtype=torch.float32, device=device)
+    return t, L.ptr(t)
+
+
+@_on_device
+def render_loss_grad(hm, joints, vis, render, reduction="mean", loss_scale=1.0, grad_scale=None, workspace=None):
+    """The fused loss and d loss / d hm in ONE pass over hm (lhn_render_loss_grad).  The gradient is the one
+    lhn_render_loss_backward computes for an upstream gradient ``grad_scale`` (float or 0-dim CUDA tensor;
+    None = 1).  Returns dict(loss f32[1], sums f64[4], weight [B, S*K], grad like hm (contiguous),
+    used_scale f32[1])."""
+    hm_v, B, Cc, H, W, sb, sc = _plane_view(hm, "heatmaps")
+    dev = hm.device
+    rp = _render_params(render["loss_mode"], render["image_size"], render["sigma"],
+                        render.get("unbiased", True), render.get("pos_value", 0.5))
+    S = rp.num_stacks
+    if Cc % S:
+        raise L.LhnError("channel count is not a multiple of the number of stacks")
+    K = Cc // S
+    joints = _f32c(joints, "joints")
+    vis = _f32c(vis, "vis")
+    if joints.dim() != 3 or joints.shape[0] != B or joints.shape[2] < 2:
+        raise L.LhnError("joints must be [B,K,>=2]")
+    if vis.dim() == 2:
+        vis = vis.unsqueeze(-1).contiguous()
+    grad = torch.empty(hm.shape, dtype=hm.dtype, device=dev)
+    weight = torch.empty((B, Cc), dtype=torch.float32, device=dev)
+    sums = torch.empty(4, dtype=torch.float64, device=dev)
+    loss = torch.empty(1, dtype=torch.float32, device=dev)
+    used = torch.empty(1, dtype=torch.float32, device=dev)
+    keep, gp = (None, None) if grad_scale is None else _scale_tensor(grad_scale, dev)
+    ws = workspace if workspace is not None else render_loss_grad_workspace(dev, B, K, S)
+    rc = L.lib().lhn_render_loss_grad(L.ptr(hm_v), L.dtype_code(hm_v), B, K, H, W, sb, sc, C.byref(rp),
+                                      L.ptr(joints), joints.shape[2], L.ptr(vis), vis.shape[2], L.ptr(weight),
+                                      L.ptr(ws), ws.numel(), L.ptr(sums), int(reduction == "sum"), float(loss_scale),
+                                      L.ptr(loss), gp, L.ptr(used), L.ptr(grad), L.stream())
+    L.check(rc, "lhn_render_loss_grad")
+    return dict(loss=loss, sums=sums, weight=weight, grad=grad, used_scale=used)
+
+
+@_on_device
+def render_loss_backward_cond(hm, joints, vis, render, sums, grad, used_scale, reduction="mean", scale=1.0,
+                              grad_out=None, recomputed=None):
+    """Backward of render_loss_grad (lhn_render_loss_backward_cond): ``grad`` is left as it is when grad_out
+    (None = 1) is bitwise the ``used_scale`` the forward assumed, else overwritten as render_loss_backward would
+    write it.  recomputed: optional int32 [1] CUDA tensor, set to 0 or 1.  Returns grad."""
+    hm_v, B, Cc, H, W, sb, sc = _plane_view(hm, "heatmaps")
+    rp = _render_params(render["loss_mode"], render["image_size"], render["sigma"],
+                        render.get("unbiased", True), render.get("pos_value", 0.5))
+    K = Cc // rp.num_stacks
+    joints = _f32c(joints, "joints")
+    vis = _f32c(vis, "vis")
+    if vis.dim() == 2:
+        vis = vis.unsqueeze(-1).contiguous()
+    if grad.shape != hm.shape or grad.dtype != hm.dtype or not grad.is_contiguous():
+        raise L.LhnError("grad must be a contiguous tensor of the heatmaps' shape and dtype")
+    if recomputed is not None and (recomputed.dtype != torch.int32 or recomputed.numel() != 1):
+        raise L.LhnError("recomputed must be an int32 tensor of one element")
+    keep, gp = _grad_out_ptr(grad_out, hm.device)
+    rc = L.lib().lhn_render_loss_backward_cond(L.ptr(hm_v), L.dtype_code(hm_v), B, K, H, W, sb, sc, C.byref(rp),
+                                               L.ptr(joints), joints.shape[2], L.ptr(vis), vis.shape[2], L.ptr(sums),
+                                               int(reduction == "sum"), float(scale), gp, L.ptr(used_scale),
+                                               L.ptr(recomputed), L.ptr(grad), L.stream())
+    L.check(rc, "lhn_render_loss_backward_cond")
+    return grad
+
+
 @_on_device
 def simdr_smoothl1_backward(out_x, out_y, tgt_x, tgt_y, weight, scale=1.0, grad_out=None):
     dt = out_x.dtype

@@ -163,6 +163,24 @@ LHN_API const char* lhn_last_cuda_error(void);
 /* Fill taps[0..ksize) with cv2.getGaussianKernel(ksize, sigma<=0, CV_64F) (host pointer). */
 LHN_API int lhn_gaussian_taps(int ksize, double* taps);
 
+/* Which code path the last K1 call of THIS host thread launched (lhn_decode_heatmap, lhn_decode_heatmap_pck,
+ * lhn_fused_render_loss_decode and their _xch variants).  Cleared on entry to every such call that reaches the
+ * launcher, filled after a successful launch; a rejected call leaves path == 0.  For tests that must know which
+ * instantiation, team geometry and copy path a shape takes; nothing in the library reads it. */
+typedef struct {
+  int32_t path;            /* 0 = nothing launched / rejected, 1 = persistent team kernel, 2 = CTA-per-plane kernel */
+  int32_t dtype;           /* LHN_F32 / LHN_BF16 / LHN_F16 */
+  int32_t flip, loss, counters;   /* flip plane present, loss fused, PCK/AUC/EPE counters fused (0/1) */
+  int32_t wc;              /* compile-time plane width of the instantiation (team: 128/64/56/32/16; CTA: 128), 0 = run-time size */
+  int32_t twc;             /* compile-time team width in warps, 0 = run-time */
+  int32_t ks;              /* compile-time DARK window: 11, or 0 = run-time */
+  int32_t team_warps, nteams, stages, sweeper_tables;   /* team kernel geometry (0 on the CTA-per-plane kernel) */
+  int32_t use_tma;         /* planes loaded by TMA bulk copies (1) or element copies (0) */
+  int32_t ctas;            /* grid size */
+  int32_t stagger_ns;      /* delay between the first loads of consecutive teams (team kernel) */
+} lhn_k1_launch_info;
+LHN_API int lhn_k1_last_launch(lhn_k1_launch_info* out);
+
 /* ---- K1: heatmap decode, optionally fused with target render + masked MSE partial sums -------
  *
  * Replaces, in ONE pass over each heatmap plane:

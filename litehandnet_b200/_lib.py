@@ -44,6 +44,7 @@ EXPORTS = [
     "lhn_render_loss_grad_workspace_bytes", "lhn_render_loss_grad", "lhn_render_loss_backward_cond",
     "lhn_simdr_smoothl1_backward", "lhn_mpii_pckh_accumulate", "lhn_region_bbox_decode", "lhn_heatmap_nms",
     "lhn_vector_nms", "lhn_refine_points", "lhn_decode_heatmap_roi", "lhn_box_nms", "lhn_render_region_wh", "lhn_dark_refine_points",
+    "lhn_k1_last_launch",
 ]
 
 
@@ -74,6 +75,12 @@ class RegionParams(C.Structure):
                 ("taps", C.c_double * MAX_TAPS)]
 
 
+class K1LaunchInfo(C.Structure):
+    """lhn_k1_launch_info: which K1 code path the last call on this thread launched (tests only)."""
+    _fields_ = [(n, C.c_int32) for n in ("path", "dtype", "flip", "loss", "counters", "wc", "twc", "ks", "team_warps",
+                                          "nteams", "stages", "sweeper_tables", "use_tma", "ctas", "stagger_ns")]
+
+
 class LhnError(RuntimeError):
     pass
 
@@ -86,6 +93,7 @@ def _declare(lib):
     lib.lhn_version.restype = C.c_int
     lib.lhn_last_cuda_error.restype = C.c_char_p
     lib.lhn_gaussian_taps.argtypes = [i32, C.POINTER(C.c_double)]
+    lib.lhn_k1_last_launch.argtypes = [C.POINTER(K1LaunchInfo)]
     lib.lhn_decode_heatmap.argtypes = [vp, vp, vp, i32, i64, i32, i32, i32, i64, i64, i64, i64, vp, vp,
                                        C.POINTER(DecodeParams), vp, vp, vp, C.POINTER(RenderParams),
                                        vp, i32, vp, i32, vp, vp, vp]

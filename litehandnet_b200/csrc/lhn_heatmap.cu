@@ -9,6 +9,10 @@
 
 namespace lhn {
 
+// what the last K1 call of this host thread launched (lhn_k1_last_launch); cleared by run_heatmap, filled by the
+// launchers of both kernels
+thread_local lhn_k1_launch_info g_k1_launch = {};
+
 // ---- the kernel --------------------------------------------------------------------------------
 template <typename T, int WT, bool FLIP, bool LOSS, int NT>
 __global__ void __launch_bounds__(NT) heatmap_plane_kernel(const __grid_constant__ HmArgs a) {
@@ -426,7 +430,16 @@ static int launch_plane_kernel(const HmArgs& a, cudaStream_t st) {
     if (e != cudaSuccess) { set_last_error(e); return LHN_ECUDA; }
   }
   kern<<<(unsigned)a.n_planes, NT, smem, st>>>(a);
-  return check_launch();
+  const int rc = check_launch();
+  if (rc == LHN_OK) {
+    lhn_k1_launch_info& r = g_k1_launch;
+    r = {};
+    r.path = 2;
+    r.dtype = std::is_same<T, float>::value ? LHN_F32 : std::is_same<T, __nv_bfloat16>::value ? LHN_BF16 : LHN_F16;
+    r.flip = FLIP; r.loss = LOSS; r.counters = a.counters != nullptr;
+    r.wc = WT; r.use_tma = a.use_tma; r.ctas = (int32_t)a.n_planes;
+  }
+  return rc;
 }
 
 template <typename T>
@@ -447,6 +460,7 @@ static int run_heatmap(HmArgs& a, int dtype, cudaStream_t st, int* used_team_ker
   const bool flip = a.hm_flip != nullptr;
   const bool loss = a.loss_mode != LHN_LOSS_NONE;
   const size_t esz = dtype == LHN_F32 ? 4 : 2;
+  g_k1_launch = {};
   // TMA bulk copies need 16-byte aligned sources and sizes
   auto aligned = [&](const void* base, int64_t sb, int64_t sc) {
     return ((uintptr_t)base % 16 == 0) && ((sb * esz) % 16 == 0) && ((sc * esz) % 16 == 0);
@@ -526,6 +540,12 @@ namespace lhn { int num_sms(); }
 // the region keeps its older size of one per team][partials of the three-launch fallback: n_planes x 4 f64]
 static const int64_t kWsHeader = 256;
 static int64_t ws_team_bytes() { return (int64_t)lhn::num_sms() * lhn::kMaxTeamsPerCta * 32; }
+
+extern "C" int lhn_k1_last_launch(lhn_k1_launch_info* out) {
+  if (!out) return LHN_EINVAL;
+  *out = lhn::g_k1_launch;
+  return LHN_OK;
+}
 
 extern "C" int64_t lhn_fused_workspace_bytes(int64_t B, int K, int num_stacks) {
   if (B < 0 || K <= 0) return 0;

@@ -1180,6 +1180,7 @@ heatmap_team_kernel(const __grid_constant__ HmArgs a) {
 // ---- host side ----------------------------------------------------------------------------------------
 int num_sms();                       // lhn_loss_render.cu: SM count of the current device, cached per device
 static int sm_count() { return num_sms(); }
+extern thread_local lhn_k1_launch_info g_k1_launch;   // lhn_heatmap.cu: lhn_k1_last_launch()
 
 template <typename T, int WC, int TWC, bool FLIP, bool LOSS, int KS>
 static int launch_one(HmArgs& a, int nteams, size_t smem, cudaStream_t st) {
@@ -1201,7 +1202,18 @@ static int launch_one(HmArgs& a, int nteams, size_t smem, cudaStream_t st) {
   cfg.attrs = at; cfg.numAttrs = a.overlap_previous ? 1 : 0;
   e = cudaLaunchKernelEx(&cfg, kern, a);
   if (e != cudaSuccess) { set_last_error(e); return LHN_ECUDA; }
-  return check_launch();
+  const int rc = check_launch();
+  if (rc == LHN_OK) {
+    lhn_k1_launch_info& r = g_k1_launch;
+    r = {};
+    r.path = 1;
+    r.dtype = sizeof(T) == 4 ? LHN_F32 : std::is_same<T, __nv_bfloat16>::value ? LHN_BF16 : LHN_F16;
+    r.flip = FLIP; r.loss = LOSS; r.counters = a.counters != nullptr;
+    r.wc = WC; r.twc = TWC; r.ks = KS;
+    r.team_warps = a.team_warps; r.nteams = nteams; r.stages = a.stages; r.sweeper_tables = a.sweeper_tables;
+    r.use_tma = a.use_tma; r.ctas = (int32_t)ctas; r.stagger_ns = a.stagger_ns;
+  }
+  return rc;
 }
 
 template <typename T, bool FLIP, bool LOSS>

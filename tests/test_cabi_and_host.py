@@ -101,6 +101,34 @@ def test_host_argument_validation_without_gpu(lib_path):
     assert lib.lhn_evaluate_pck_workspace_bytes(64, 21) == 2 * 64 * 21 * 12
 
 
+def test_k1_launch_record_without_gpu(lib_path):
+    """lhn_k1_last_launch: a null pointer is refused; the record is per host thread, so a fresh thread reads
+    path == 0 whatever ran before, and a call rejected before the launch (misaligned plane pointer) leaves it so."""
+    import threading
+    from litehandnet_b200 import _lib
+    lib = _lib.lib()
+    assert hasattr(lib, "lhn_k1_last_launch")
+    assert ctypes.sizeof(_lib.K1LaunchInfo) == 15 * 4
+    assert lib.lhn_k1_last_launch(None) == -1
+    seen = []
+
+    def probe():
+        r = _lib.K1LaunchInfo()
+        r.path, r.ctas = 7, 7
+        seen.append((lib.lhn_k1_last_launch(ctypes.byref(r)), r.path, r.ctas))
+        dp = _lib.DecodeParams()
+        rc = lib.lhn_decode_heatmap(ctypes.c_void_p(18), None, None, _lib.F32, 1, 21, 64, 64, 21 * 4096, 4096, 0, 0,
+                                    None, None, ctypes.byref(dp), None, None, None, None, None, 0, None, 0, None, None,
+                                    None)
+        r.path = 7
+        seen.append((rc, lib.lhn_k1_last_launch(ctypes.byref(r)), r.path))
+
+    t = threading.Thread(target=probe)
+    t.start()
+    t.join()
+    assert seen == [(0, 0, 0), (-3, 0, 0)], seen
+
+
 def test_no_cpu_fallback():
     """CPU tensors are refused loudly; nothing under litehandnet_b200/ imports the oracle."""
     from litehandnet_b200 import _lib, ops

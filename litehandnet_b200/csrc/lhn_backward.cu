@@ -86,14 +86,7 @@ __global__ void __launch_bounds__(128) render_loss_backward_kernel(const __grid_
                                    a.feat_x, a.feat_y, 0, 0.0, 0.0, W, H);
   float w = g.w;
   const double inv2s2 = 1.0 / (2.0 * sig * sig);
-  for (int i = threadIdx.x; i < W + H; i += blockDim.x) {
-    float v = 0.f;
-    if (g.on) {
-      const double arg = render_arg(g, i, W, a.unbiased, inv2s2);
-      if (arg <= 0.0) v = exp_f32_from_f64(arg);         // as the forward kernel evaluates it
-    }
-    tab[i] = v;
-  }
+  for (int i = threadIdx.x; i < W + H; i += blockDim.x) tab[i] = table_entry(g, i, W, a.unbiased, inv2s2);
   float cpos, cneg;
   loss_coefs(a.sums, a.loss_mode, a.sum_reduction, a.scale, a.grad_out, cpos, cneg);
   if (a.loss_mode == LHN_LOSS_JOINTS_MSE) w *= w;

@@ -136,8 +136,8 @@ __device__ __forceinline__ float warp_sum(float v) {
 
 // ---------------------------------------------------------------------------------------------
 // Gaussian target geometry (generateTarget.py:100-154 MSRA, :162-243 UDP), shared by the fused kernel,
-// the CTA-per-plane fallback, lhn_render_targets and the backward kernel so that all four render the
-// same target.  mode = lhn_render_params.unbiased: 1 = MSRA sub-pixel full plane, 0 = MSRA integer
+// the CTA-per-plane fallback, lhn_render_targets, the two-pass backward and the one-pass loss + gradient so
+// that all five render the same target.  mode = lhn_render_params.unbiased: 1 = MSRA sub-pixel full plane, 0 = MSRA integer
 // centre patch, 2 = UDP (integer patch position, sub-pixel Gaussian centre inside it).
 // ---------------------------------------------------------------------------------------------
 struct RenderGeom {
@@ -201,6 +201,16 @@ __device__ __forceinline__ float exp_f32_from_f64(double a) {
   const float al = (float)(a - (double)ah);
   const float v = expf(ah);
   return fmaf(v, al, v);
+}
+
+// Table entry i (i < W: x table, else y table) of the separable Gaussian: the one definition every kernel that
+// renders the target calls, so that they all draw the same bits.  0 on a plane without a Gaussian and outside the
+// patch (arg = +1).  `!(arg > 0)` passes a NaN argument (a NaN joint in mode 1) through as NaN, as the reference's
+// np.exp does: the plane's target is NaN rather than silently 0.
+__device__ __forceinline__ float table_entry(const RenderGeom& g, int i, int W, int mode, double inv2s2) {
+  if (!g.on) return 0.f;
+  const double arg = render_arg(g, i, W, mode, inv2s2);
+  return !(arg > 0.0) ? exp_f32_from_f64(arg) : 0.f;
 }
 
 // ---------------------------------------------------------------------------------------------

@@ -86,14 +86,7 @@ __global__ void __launch_bounds__(NT) heatmap_plane_kernel(const __grid_constant
     render_on = g.on;
     gcx = g.cx; gcy = g.cy;
     const double inv2s2 = 1.0 / (2.0 * sig * sig);
-    for (int i = tid; i < W + H; i += NT) {
-      float v = 0.f;
-      if (render_on) {
-        const double arg = render_arg(g, i, W, a.unbiased, inv2s2);
-        if (arg <= 0.0) v = (float)exp(arg);
-      }
-      ex[i] = v;   // ey follows ex contiguously
-    }
+    for (int i = tid; i < W + H; i += NT) ex[i] = table_entry(g, i, W, a.unbiased, inv2s2);   // ey follows ex
   }
   __syncthreads();   // tables (and the non-TMA copy) visible
   if (a.use_tma) mbar_wait(&sh->bar, 0);

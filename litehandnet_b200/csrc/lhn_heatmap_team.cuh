@@ -310,11 +310,7 @@ heatmap_team_kernel(const __grid_constant__ HmArgs a) {
     }
     const double i2 = a.inv2s2[s];
     float* tab = reinterpret_cast<float*>(reinterpret_cast<unsigned char*>(tab0) + (size_t)buf * tab_bytes);
-    auto entry = [&](int i) -> float {
-      const double arg = render_arg(g, i, W, a.unbiased, i2);
-      const float v = arg <= 0.0 ? exp_f32_from_f64(arg) : 0.f;
-      return render_on ? v : 0.f;
-    };
+    auto entry = [&](int i) -> float { return table_entry(g, i, W, a.unbiased, i2); };
     // four independent f64 chains per thread at a time: the loop is latency-bound, not throughput-bound
     const int n = W + H;
     int i0 = t;

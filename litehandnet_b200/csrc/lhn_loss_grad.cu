@@ -151,13 +151,6 @@ __device__ __forceinline__ PlaneRec plane_rec(const LossGradArgs& a, int64_t p) 
   return r;
 }
 
-// table entry i (i < W: x, else y): exactly the value the fused forward and the two-pass backward evaluate
-__device__ __forceinline__ float table_entry(const RenderGeom& g, int i, int W, int mode, double inv2s2) {
-  if (!g.on) return 0.f;
-  const double arg = render_arg(g, i, W, mode, inv2s2);
-  return arg <= 0.0 ? exp_f32_from_f64(arg) : 0.f;
-}
-
 __device__ __forceinline__ const void* plane_src(const LossGradArgs& a, int64_t p, size_t esz) {
   const PlaneIdx q = plane_idx(a, p);
   return reinterpret_cast<const unsigned char*>(a.hm) + (size_t)(q.b * a.stride_b + (int64_t)q.c * a.stride_c) * esz;

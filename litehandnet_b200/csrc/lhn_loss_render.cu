@@ -166,14 +166,7 @@ __global__ void __launch_bounds__(128) render_targets_kernel(const __grid_consta
                                    a.feat_x, a.feat_y, 0, 0.0, 0.0, W, H);
   const float w = g.w;
   const double inv2s2 = 1.0 / (2.0 * sig * sig);
-  for (int i = threadIdx.x; i < W + H; i += blockDim.x) {
-    float v = 0.f;
-    if (g.on) {
-      const double arg = render_arg(g, i, W, a.unbiased, inv2s2);
-      if (arg <= 0.0) v = (float)exp(arg);
-    }
-    tab[i] = v;
-  }
+  for (int i = threadIdx.x; i < W + H; i += blockDim.x) tab[i] = table_entry(g, i, W, a.unbiased, inv2s2);
   __syncthreads();
   float* dst = a.target + p * (int64_t)H * W;
   if ((W & 3) == 0) {

@@ -181,6 +181,26 @@ typedef struct {
 } lhn_k1_launch_info;
 LHN_API int lhn_k1_last_launch(lhn_k1_launch_info* out);
 
+/* Which code path the last SimDR call of THIS host thread launched (lhn_render_simdr(_f64sigma), lhn_decode_simdr(_flags),
+ * lhn_simdr_smoothl1, lhn_simdr_smoothl1_backward, lhn_simdr_heads_loss(_f32)).  Cleared on entry to each of them,
+ * filled after a successful launch; a rejected call leaves family == 0.  For tests that must know which kernel and
+ * geometry a shape takes; nothing in the library reads it. */
+typedef struct {
+  int32_t family;          /* 0 = nothing launched / rejected, 1 render, 2 decode, 3 loss, 4 backward, 5 heads */
+  int32_t path;            /* render: 1 windowed (warp per joint), 2 plain (CTA per joint);
+                              decode: 1 TMA ring, 2 pair scan, 3 scalar scan, 4 NMS;
+                              loss: 1 joint-per-warp + cluster finalise, 2 rows + cluster finalise,
+                                    3 rows + one-block finalise, 4 rows + single-thread loop (K > 1024);
+                              backward, heads: 1 */
+  int32_t dtype;           /* LHN_F32 / LHN_BF16 / LHN_F16 of the vectors (heads: LHN_BF16 operands) */
+  int32_t warps;           /* warps per CTA of the main kernel */
+  int32_t stages;          /* decode ring / heads mbarrier ring stages, else 0 */
+  int32_t ctas;            /* grid size of the main kernel */
+  int32_t vec_x, vec_y;    /* 128-bit path over the x / y vectors (backward per vector; loss: one flag for both) */
+  int32_t bn;              /* heads: N tile width, else 0 */
+} lhn_simdr_launch_info;
+LHN_API int lhn_simdr_last_launch(lhn_simdr_launch_info* out);
+
 /* ---- K1: heatmap decode, optionally fused with target render + masked MSE partial sums -------
  *
  * Replaces, in ONE pass over each heatmap plane:
@@ -361,10 +381,18 @@ LHN_API int lhn_render_targets(const float* joints, int joints_stride, const flo
                                lhn_stream_t stream);
 
 /* GenerateSimDR._generate_sa_simdr (generate_simder.py:9-31): simdr_x f32 [B,K,Lx],
- * simdr_y f32 [B,K,Ly]; Lx = int(image_w*k), Ly = int(image_h*k). */
+ * simdr_y f32 [B,K,Ly]; Lx = int(image_w*k), Ly = int(image_h*k).  The Gaussian's denominator is
+ * 2.f * sigma * sigma in f32 arithmetic. */
 LHN_API int lhn_render_simdr(const float* joints, int joints_stride, const float* vis,
                              int vis_stride, int64_t B, int K, int Lx, int Ly, float split_ratio,
                              float sigma, float* simdr_x, float* simdr_y, lhn_stream_t stream);
+/* The same with sigma as a double, bit for bit the reference: it divides by the Python float
+ * 2 * sigma ** 2, formed in f64 and rounded to f32 once, and this entry point forms
+ * (float)(2.0 * sigma * sigma) the same way.  An f32 sigma cannot reproduce that denominator: for about
+ * half of all sigma (1.3, 2.1, 2.7, 3.3, ...) 2.f * s * s is one f32 ulp away from it. */
+LHN_API int lhn_render_simdr_f64sigma(const float* joints, int joints_stride, const float* vis,
+                                      int vis_stride, int64_t B, int K, int Lx, int Ly, float split_ratio,
+                                      double sigma, float* simdr_x, float* simdr_y, lhn_stream_t stream);
 
 /* ---- K2: SimDR --------------------------------------------------------------------------------
  * keypoints_from_simdr (top_down_eval.py:466-500): x = argmax(x_vec)/k, y = argmax(y_vec)/k,

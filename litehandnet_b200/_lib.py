@@ -35,7 +35,7 @@ ERRORS = {-1: "LHN_EINVAL (bad shape / null pointer / bad enum)", -2: "LHN_EDTYP
 EXPORTS = [
     "lhn_version", "lhn_last_cuda_error", "lhn_gaussian_taps", "lhn_decode_heatmap",
     "lhn_decode_heatmap_pck", "lhn_loss_partials", "lhn_loss_reduce", "lhn_loss_finalize", "lhn_loss_mse_workspace_bytes", "lhn_loss_mse_multi",
-    "lhn_render_targets", "lhn_render_simdr", "lhn_decode_simdr", "lhn_decode_simdr_flags", "lhn_simdr_loss_workspace_bytes",
+    "lhn_render_targets", "lhn_render_simdr", "lhn_render_simdr_f64sigma", "lhn_decode_simdr", "lhn_decode_simdr_flags", "lhn_simdr_loss_workspace_bytes",
     "lhn_simdr_smoothl1", "lhn_split_bf16", "lhn_simdr_heads_workspace_bytes", "lhn_simdr_heads_loss",
     "lhn_simdr_heads_f32_workspace_bytes", "lhn_simdr_heads_loss_f32", "lhn_pck_accumulate", "lhn_metrics_finalize", "lhn_evaluate_pck_workspace_bytes",
     "lhn_evaluate_pck", "lhn_flip_back", "lhn_fused_workspace_bytes", "lhn_fused_render_loss_decode",
@@ -44,7 +44,7 @@ EXPORTS = [
     "lhn_render_loss_grad_workspace_bytes", "lhn_render_loss_grad", "lhn_render_loss_backward_cond",
     "lhn_simdr_smoothl1_backward", "lhn_mpii_pckh_accumulate", "lhn_region_bbox_decode", "lhn_heatmap_nms",
     "lhn_vector_nms", "lhn_refine_points", "lhn_decode_heatmap_roi", "lhn_box_nms", "lhn_render_region_wh", "lhn_dark_refine_points",
-    "lhn_k1_last_launch",
+    "lhn_k1_last_launch", "lhn_simdr_last_launch",
 ]
 
 
@@ -81,6 +81,11 @@ class K1LaunchInfo(C.Structure):
                                           "nteams", "stages", "sweeper_tables", "use_tma", "ctas", "stagger_ns")]
 
 
+class SimdrLaunchInfo(C.Structure):
+    """lhn_simdr_launch_info: which SimDR kernel and geometry the last SimDR call on this thread launched (tests only)."""
+    _fields_ = [(n, C.c_int32) for n in ("family", "path", "dtype", "warps", "stages", "ctas", "vec_x", "vec_y", "bn")]
+
+
 class LhnError(RuntimeError):
     pass
 
@@ -94,6 +99,7 @@ def _declare(lib):
     lib.lhn_last_cuda_error.restype = C.c_char_p
     lib.lhn_gaussian_taps.argtypes = [i32, C.POINTER(C.c_double)]
     lib.lhn_k1_last_launch.argtypes = [C.POINTER(K1LaunchInfo)]
+    lib.lhn_simdr_last_launch.argtypes = [C.POINTER(SimdrLaunchInfo)]
     lib.lhn_decode_heatmap.argtypes = [vp, vp, vp, i32, i64, i32, i32, i32, i64, i64, i64, i64, vp, vp,
                                        C.POINTER(DecodeParams), vp, vp, vp, C.POINTER(RenderParams),
                                        vp, i32, vp, i32, vp, vp, vp]
@@ -137,6 +143,7 @@ def _declare(lib):
     lib.lhn_render_targets.argtypes = [vp, i32, vp, i32, i64, i32, i32, i32, C.POINTER(RenderParams),
                                        vp, vp, vp]
     lib.lhn_render_simdr.argtypes = [vp, i32, vp, i32, i64, i32, i32, i32, f32, f32, vp, vp, vp]
+    lib.lhn_render_simdr_f64sigma.argtypes = [vp, i32, vp, i32, i64, i32, i32, i32, f32, f64, vp, vp, vp]
     lib.lhn_decode_simdr.argtypes = [vp, vp, i32, i64, i32, i32, i32, i32, vp, vp, i32, vp, vp, vp, vp]
     lib.lhn_decode_simdr_flags.argtypes = [vp, vp, i32, i64, i32, i32, i32, i32, vp, vp, i32, vp, vp, vp, i32, vp]
     lib.lhn_simdr_loss_workspace_bytes.argtypes = [i64, i32]

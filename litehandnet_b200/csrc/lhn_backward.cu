@@ -253,6 +253,7 @@ extern "C" int lhn_simdr_smoothl1_backward(const void* out_x, const void* out_y,
                                            int Lx, int Ly, float scale, const float* grad_out, void* workspace,
                                            int64_t workspace_bytes, void* grad_x, void* grad_y,
                                            lhn_stream_t stream) {
+  g_simdr_launch = {};
   if (!out_x || !out_y || !tgt_x || !tgt_y || !weight || !workspace || !grad_x || !grad_y || B <= 0 || K <= 0 ||
       Lx <= 0 || Ly <= 0)
     return LHN_EINVAL;
@@ -275,5 +276,13 @@ extern "C" int lhn_simdr_smoothl1_backward(const void* out_x, const void* out_y,
     default: return LHN_EDTYPE;
   }
 #undef LHN_SB
-  return check_launch();
+  const int rc = check_launch();
+  if (rc == LHN_OK) {
+    // the kernel's per-row `vec` test: with L % 4 == 0 every row of an aligned base is aligned
+    const uintptr_t al = dtype == LHN_F32 ? 16 : 8;
+    const bool vx = (Lx & 3) == 0 && (((uintptr_t)out_x | (uintptr_t)tgt_x | (uintptr_t)grad_x) % al) == 0;
+    const bool vy = (Ly & 3) == 0 && (((uintptr_t)out_y | (uintptr_t)tgt_y | (uintptr_t)grad_y) % al) == 0;
+    simdr_record(4, 1, dtype, threads / 32, 0, nb, vx, vy, 0);
+  }
+  return rc;
 }

@@ -8,6 +8,15 @@
 #include "../../include/lhn.h"
 
 namespace lhn {
+// what the last SimDR call of this host thread launched (lhn_simdr_last_launch; defined in lhn_simdr.cu)
+extern thread_local lhn_simdr_launch_info g_simdr_launch;
+inline void simdr_record(int family, int path, int dtype, int warps, int stages, int64_t ctas, int vec_x, int vec_y,
+                         int bn) {
+  g_simdr_launch = lhn_simdr_launch_info{family, path, dtype, warps, stages, (int32_t)ctas, vec_x, vec_y, bn};
+}
+}  // namespace lhn
+
+namespace lhn {
 
 constexpr int kWarp = 32;
 

@@ -207,9 +207,8 @@ template <bool VEC>
 __global__ void __launch_bounds__(256) render_simdr_kernel(const float* __restrict__ joints, int js,
                                                            const float* __restrict__ vis, int vs,
                                                            int64_t n_bk, int Lx, int Ly, float kf,
-                                                           float sigma, float* __restrict__ sx,
+                                                           float den, float* __restrict__ sx,
                                                            float* __restrict__ sy) {
-  const float den = 2.f * sigma * sigma;
   if (VEC) {
     __shared__ float win_all[8][kSimdrWindowMax];
     const int lane = threadIdx.x & 31;
@@ -370,23 +369,47 @@ extern "C" int lhn_render_targets(const float* joints, int joints_stride, const 
   return check_launch();
 }
 
-extern "C" int lhn_render_simdr(const float* joints, int joints_stride, const float* vis,
-                                int vis_stride, int64_t B, int K, int Lx, int Ly, float split_ratio,
-                                float sigma, float* simdr_x, float* simdr_y, lhn_stream_t stream) {
+// Both render entry points: `den` is the Gaussian's denominator 2 sigma^2 as an f32, formed by the caller.
+static int render_simdr_den(const float* joints, int joints_stride, const float* vis, int vis_stride, int64_t B, int K,
+                            int Lx, int Ly, float split_ratio, float den, float* simdr_x, float* simdr_y,
+                            lhn_stream_t stream) {
   if (!joints || !vis || !simdr_x || !simdr_y || B < 0 || K <= 0 || Lx <= 0 || Ly <= 0 ||
-      joints_stride < 2 || vis_stride < 1 || !(sigma > 0.f))
+      joints_stride < 2 || vis_stride < 1 || !(den > 0.f) || !(den <= 3.4028235e38f))
     return LHN_EINVAL;
   const int64_t n = B * K;
   if (n == 0) return LHN_OK;
   if (n > 0x7fffffffLL) return LHN_EINVAL;
   const bool vec = Lx % 4 == 0 && Ly % 4 == 0 && ((uintptr_t)simdr_x % 16) == 0 && ((uintptr_t)simdr_y % 16) == 0 &&
-                   2 * (int)ceilf(sqrtf(104.f * 2.f * sigma * sigma) + 1.f) + 2 <= kSimdrWindowMax;
+                   2 * (int)ceilf(sqrtf(104.f * den) + 1.f) + 2 <= kSimdrWindowMax;
   const int64_t want = (n + 7) / 8, cap = (int64_t)num_sms() * 8;
-  if (vec) render_simdr_kernel<true><<<(unsigned)(want < cap ? want : cap), 256, 0, (cudaStream_t)stream>>>(joints, joints_stride, vis, vis_stride,
-      n, Lx, Ly, split_ratio, sigma, simdr_x, simdr_y);
-  else render_simdr_kernel<false><<<(unsigned)n, 256, 0, (cudaStream_t)stream>>>(joints, joints_stride, vis, vis_stride,
-      n, Lx, Ly, split_ratio, sigma, simdr_x, simdr_y);
-  return check_launch();
+  const int64_t ctas = vec ? (want < cap ? want : cap) : n;
+  if (vec) render_simdr_kernel<true><<<(unsigned)ctas, 256, 0, (cudaStream_t)stream>>>(joints, joints_stride, vis, vis_stride,
+      n, Lx, Ly, split_ratio, den, simdr_x, simdr_y);
+  else render_simdr_kernel<false><<<(unsigned)ctas, 256, 0, (cudaStream_t)stream>>>(joints, joints_stride, vis, vis_stride,
+      n, Lx, Ly, split_ratio, den, simdr_x, simdr_y);
+  const int rc = check_launch();
+  if (rc == LHN_OK) simdr_record(1, vec ? 1 : 2, LHN_F32, 8, 0, ctas, vec, vec, 0);
+  return rc;
+}
+
+extern "C" int lhn_render_simdr(const float* joints, int joints_stride, const float* vis,
+                                int vis_stride, int64_t B, int K, int Lx, int Ly, float split_ratio,
+                                float sigma, float* simdr_x, float* simdr_y, lhn_stream_t stream) {
+  g_simdr_launch = {};
+  if (!(sigma > 0.f)) return LHN_EINVAL;
+  return render_simdr_den(joints, joints_stride, vis, vis_stride, B, K, Lx, Ly, split_ratio, 2.f * sigma * sigma,
+                          simdr_x, simdr_y, stream);
+}
+
+extern "C" int lhn_render_simdr_f64sigma(const float* joints, int joints_stride, const float* vis,
+                                         int vis_stride, int64_t B, int K, int Lx, int Ly, float split_ratio,
+                                         double sigma, float* simdr_x, float* simdr_y, lhn_stream_t stream) {
+  g_simdr_launch = {};
+  if (!(sigma > 0.0)) return LHN_EINVAL;
+  // the reference's denominator: the Python float 2 * sigma ** 2 (f64), rounded to f32 once when numpy divides the f32
+  // array by it.  2.f * s * s on an f32 sigma differs from it by one ulp for about half of all sigma (1.3, 2.1, 2.7, ...)
+  return render_simdr_den(joints, joints_stride, vis, vis_stride, B, K, Lx, Ly, split_ratio,
+                          (float)(2.0 * (sigma * sigma)), simdr_x, simdr_y, stream);
 }
 
 extern "C" int lhn_flip_back(const void* in, void* out, int dtype, int64_t B, int K, int H, int W,

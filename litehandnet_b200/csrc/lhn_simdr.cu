@@ -10,13 +10,18 @@
 namespace lhn {
 int num_sms();
 
+thread_local lhn_simdr_launch_info g_simdr_launch = {};
+
 // first-max argmax of one vector by one warp; NaN is maximal.
 // NMS: value kept iff it equals max(v[i-1], v[i], v[i+1]) (max_pool1d k=3,s=1,p=1 with -inf
 // padding) else 0; then multiplied by the [lo, hi) mask (result_parser.py:61-74,113-121).
+// The value reported is the selected element itself (after NMS and the mask), as numpy's take_along_axis gives it:
+// −0 and +0 tie (the key maps both to +0) but the score keeps the sign of the element at the first index.
 template <typename T, bool NMS>
 __device__ __forceinline__ void warp_vec_argmax(const T* __restrict__ v, int L, int lo, int hi,
                                                 int lane, uint32_t& out_idx, float& out_val) {
   uint32_t bkey = 0u, bidx = 0xffffffffu;
+  float bval = 0.f;                                          // this lane's first element of key bkey
   const bool vec = ((L & 3) == 0) && (reinterpret_cast<uintptr_t>(v) % (4 * sizeof(T)) == 0);
   if (vec && !NMS) {
     const int nq = L >> 2;
@@ -36,8 +41,8 @@ __device__ __forceinline__ void warp_vec_argmax(const T* __restrict__ v, int L, 
         else if (a.w != a.w) { has_nan = true; nan_idx = e + 3; }
       }
     }
-    if (has_nan) { bkey = 0xffffffffu; bidx = nan_idx; }
-    else bkey = order_key(best);
+    if (has_nan) { bkey = 0xffffffffu; bidx = nan_idx; bval = CUDART_NAN_F; }
+    else { bkey = order_key(best); bval = best; }
   } else {
     // scalar path (also the NMS path: neighbours via an overlapping read)
     for (int i = lane; i < L; i += 32) {
@@ -52,15 +57,16 @@ __device__ __forceinline__ void warp_vec_argmax(const T* __restrict__ v, int L, 
         x = x * ((i >= lo && i < hi) ? 1.f : 0.f);
       }
       const uint32_t kx = order_key(x);
-      if (bidx == 0xffffffffu || kx > bkey) { bkey = kx; bidx = (uint32_t)i; }
+      if (bidx == 0xffffffffu || kx > bkey) { bkey = kx; bidx = (uint32_t)i; bval = x; }
     }
     if (bidx == 0xffffffffu) bkey = 0u;
   }
-  if (bidx == 0xffffffffu && bkey != 0xffffffffu) { /* lane saw nothing or only -inf */ }
   warp_argmax(bkey, bidx);
   if (bidx == 0xffffffffu) bidx = 0;
   out_idx = bidx;
-  out_val = key_to_float(bkey);
+  // the lane that scanned element bidx holds it as its own first maximum
+  const int src = (vec && !NMS) ? (int)((bidx >> 2) & 31u) : (int)(bidx & 31u);
+  out_val = __shfl_sync(0xffffffffu, bval, src);
 }
 
 // Fast path (no NMS, 16-byte aligned vectors): both vectors of a (b, k) pair are scanned in ONE loop so that all
@@ -527,7 +533,7 @@ simdr_loss_finalize_cluster_kernel(const double* __restrict__ per_bk, const floa
 }
 
 template <typename T>
-static int launch_simdr(const void* xv, const void* yv, int64_t n_bk, int K, int Lx, int Ly, int k,
+static int launch_simdr(int dtype, const void* xv, const void* yv, int64_t n_bk, int K, int Lx, int Ly, int k,
                         const float* center, const float* scale, int nms, const int32_t* ranges,
                         float* out, int32_t* out_idx, int flags, cudaStream_t st) {
   // Ring kernel: no NMS, TMA-able vectors (16-byte multiples, 16-byte aligned bases), at least two stages per warp,
@@ -562,7 +568,9 @@ static int launch_simdr(const void* xv, const void* yv, int64_t n_bk, int K, int
       e = cudaLaunchKernelEx(&cfg, decode_simdr_ring_kernel<T>, (const T*)xv, (const T*)yv, n_bk, K, Lx, Ly, k, center, scale,
                              out, out_idx, nstg, (int)pair_al, overlap);
       if (e != cudaSuccess) { set_last_error(e); return LHN_ECUDA; }
-      return check_launch();
+      const int rc = check_launch();
+      if (rc == LHN_OK) simdr_record(2, 1, dtype, warps, nstg, num_sms(), 1, 1, 0);
+      return rc;
     }
   }
   const int threads = 256;
@@ -575,7 +583,15 @@ static int launch_simdr(const void* xv, const void* yv, int64_t n_bk, int K, int
   else
     decode_simdr_kernel<T, false><<<blocks, threads, 0, st>>>((const T*)xv, (const T*)yv, n_bk, K, Lx, Ly, k,
                                                               center, scale, ranges, out, out_idx);
-  return check_launch();
+  const int rc = check_launch();
+  if (rc == LHN_OK) {
+    // the kernel's per-pair `fast` test: every row of an aligned base with L % 4 == 0 is aligned as well
+    const bool fast = ((Lx | Ly) & 3) == 0 && ((reinterpret_cast<uintptr_t>(xv) | reinterpret_cast<uintptr_t>(yv)) %
+                                              (4 * sizeof(T))) == 0;
+    const int path = nms ? 4 : (fast ? 2 : 3);
+    simdr_record(2, path, dtype, threads / 32, 0, blocks, path == 2, path == 2, 0);
+  }
+  return rc;
 }
 
 }  // namespace lhn
@@ -594,6 +610,7 @@ extern "C" int lhn_decode_simdr_flags(const void* x_vec, const void* y_vec, int 
                                       int Lx, int Ly, int split_ratio, const float* center,
                                       const float* scale, int nms, const int32_t* ranges, float* out,
                                       int32_t* out_idx, int flags, lhn_stream_t stream) {
+  g_simdr_launch = {};
   if (!x_vec || !y_vec || !out || B < 0 || K <= 0 || Lx <= 0 || Ly <= 0 || split_ratio <= 0 ||
       ((center == nullptr) != (scale == nullptr)))
     return LHN_EINVAL;
@@ -601,11 +618,17 @@ extern "C" int lhn_decode_simdr_flags(const void* x_vec, const void* y_vec, int 
   if (n == 0) return LHN_OK;
   cudaStream_t st = (cudaStream_t)stream;
   switch (dtype) {
-    case LHN_F32: return launch_simdr<float>(x_vec, y_vec, n, K, Lx, Ly, split_ratio, center, scale, nms, ranges, out, out_idx, flags, st);
-    case LHN_BF16: return launch_simdr<__nv_bfloat16>(x_vec, y_vec, n, K, Lx, Ly, split_ratio, center, scale, nms, ranges, out, out_idx, flags, st);
-    case LHN_F16: return launch_simdr<__half>(x_vec, y_vec, n, K, Lx, Ly, split_ratio, center, scale, nms, ranges, out, out_idx, flags, st);
+    case LHN_F32: return launch_simdr<float>(dtype, x_vec, y_vec, n, K, Lx, Ly, split_ratio, center, scale, nms, ranges, out, out_idx, flags, st);
+    case LHN_BF16: return launch_simdr<__nv_bfloat16>(dtype, x_vec, y_vec, n, K, Lx, Ly, split_ratio, center, scale, nms, ranges, out, out_idx, flags, st);
+    case LHN_F16: return launch_simdr<__half>(dtype, x_vec, y_vec, n, K, Lx, Ly, split_ratio, center, scale, nms, ranges, out, out_idx, flags, st);
     default: return LHN_EDTYPE;
   }
+}
+
+extern "C" int lhn_simdr_last_launch(lhn_simdr_launch_info* out) {
+  if (!out) return LHN_EINVAL;
+  *out = g_simdr_launch;
+  return LHN_OK;
 }
 
 extern "C" int64_t lhn_simdr_loss_workspace_bytes(int64_t B, int K) {
@@ -617,6 +640,7 @@ extern "C" int lhn_simdr_smoothl1(const void* out_x, const void* out_y, const vo
                                   const void* tgt_y, const float* weight, int dtype, int64_t B, int K,
                                   int Lx, int Ly, void* workspace, int64_t workspace_bytes, float* loss,
                                   lhn_stream_t stream) {
+  g_simdr_launch = {};
   if (!out_x || !out_y || !tgt_x || !tgt_y || !weight || !workspace || !loss || B <= 0 || K <= 0 ||
       Lx <= 0 || Ly <= 0)
     return LHN_EINVAL;
@@ -628,7 +652,10 @@ extern "C" int lhn_simdr_smoothl1(const void* out_x, const void* out_y, const vo
   int blocks = (int)(need < cap ? need : cap);
   cudaStream_t st = (cudaStream_t)stream;
   double* per_bk = (double*)workspace;
-  static const int mode = [] { const char* e = getenv("LHN_SIMDR_LOSS_PATH"); return e ? atoi(e) : 0; }();   // 1: rows + one block, 2: rows + cluster
+  // read on every call, like LHN_SIMDR_RING / LHN_SIMDR_WARPS: 1 = rows + one block, 2 = rows + cluster (where the shape
+  // allows the cluster finalise; otherwise rows + one block)
+  const char* mode_env = getenv("LHN_SIMDR_LOSS_PATH");
+  const int mode = mode_env ? atoi(mode_env) : 0;
   const size_t es = dtype == LHN_F32 ? 4 : 2;
   const bool vec = ((Lx | Ly) & 3) == 0 && (((uintptr_t)out_x | (uintptr_t)out_y | (uintptr_t)tgt_x | (uintptr_t)tgt_y) % (4 * es)) == 0;
   auto finalize_cluster = [&](const float* w, int64_t entries) -> int {
@@ -682,7 +709,9 @@ extern "C" int lhn_simdr_smoothl1(const void* out_x, const void* out_y, const vo
       }
       int rc = check_launch();
       if (rc) return rc;
-      return finalize_cluster(nullptr, warps);
+      rc = finalize_cluster(nullptr, warps);
+      if (rc == LHN_OK) simdr_record(3, 1, dtype, threads / 32, 0, jb, 1, 1, 0);
+      return rc;
     }
   }
   switch (dtype) {
@@ -702,7 +731,14 @@ extern "C" int lhn_simdr_smoothl1(const void* out_x, const void* out_y, const vo
   }
   int rc = check_launch();
   if (rc) return rc;
-  if (K <= kFinClusterMaxK && n >= 8192 && mode != 1) return finalize_cluster(weight, n);
+  if (K <= kFinClusterMaxK && n >= 8192 && mode != 1) {
+    rc = finalize_cluster(weight, n);
+    if (rc == LHN_OK) simdr_record(3, 2, dtype, threads / 32, 0, blocks, vec, vec, 0);
+    return rc;
+  }
   simdr_loss_finalize_kernel<<<1, 1024, 0, st>>>(per_bk, weight, B, K, Lx, Ly, loss);
-  return check_launch();
+  rc = check_launch();
+  // the finalise walks the joints in one thread when they outnumber its 1024 threads
+  if (rc == LHN_OK) simdr_record(3, K > 1024 ? 4 : 3, dtype, threads / 32, 0, blocks, vec, vec, 0);
+  return rc;
 }

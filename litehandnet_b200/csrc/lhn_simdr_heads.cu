@@ -216,8 +216,9 @@ simdr_heads_kernel(const __grid_constant__ CUtensorMap tm_ahi, const __grid_cons
           const float s4 = (smooth_l1_f(d.x) + smooth_l1_f(d.y)) + (smooth_l1_f(d.z) + smooth_l1_f(d.w));
           if (isx) sx += s4; else sy += s4;
           if (a.dpred) {
-            const float4 g = make_float4(fminf(fmaxf(d.x, -1.f), 1.f), fminf(fmaxf(d.y, -1.f), 1.f),
-                                         fminf(fmaxf(d.z, -1.f), 1.f), fminf(fmaxf(d.w, -1.f), 1.f));
+            // clamp that keeps NaN, as torch's clamp and the SmoothL1 gradient do (fmaxf alone would return -1)
+            auto clamp1 = [](float v) { return v != v ? v : fminf(fmaxf(v, -1.f), 1.f); };
+            const float4 g = make_float4(clamp1(d.x), clamp1(d.y), clamp1(d.z), clamp1(d.w));
             *reinterpret_cast<float4*>(a.dpred + (size_t)row * a.N + col) = g;
           }
           if (a.pred) *reinterpret_cast<float4*>(a.pred + (size_t)row * a.N + col) = p;
@@ -378,6 +379,7 @@ extern "C" int lhn_simdr_heads_loss_f32(const float* heatmap, const void* w_hi, 
                                         const float* target_x, const float* target_y, const float* weight, int64_t B,
                                         int K, int Kd, int Lx, int Ly, void* workspace, int64_t workspace_bytes,
                                         float* loss, float* dpred, float* pred, lhn_stream_t stream) {
+  g_simdr_launch = {};
   if (!heatmap || !workspace || B <= 0 || K <= 0 || Kd <= 0 || (Kd & 3)) return LHN_EINVAL;
   const int64_t need = lhn_simdr_heads_f32_workspace_bytes(B, K, Kd, Lx, Ly);
   if (need < 0) return LHN_EINVAL;
@@ -398,6 +400,7 @@ extern "C" int lhn_simdr_heads_loss(const void* a_hi, const void* a_lo, const vo
                                     const float* weight, int64_t B, int K, int Kd, int Lx, int Ly, void* workspace,
                                     int64_t workspace_bytes, float* loss, float* dpred, float* pred,
                                     lhn_stream_t stream) {
+  g_simdr_launch = {};
   if (!a_hi || !a_lo || !w_hi || !w_lo || !bias || !target_x || !target_y || !weight || !workspace || !loss || B <= 0 ||
       K <= 0 || Kd <= 0 || Lx <= 0 || Ly <= 0)
     return LHN_EINVAL;
@@ -423,5 +426,10 @@ extern "C" int lhn_simdr_heads_loss(const void* a_hi, const void* a_lo, const vo
                      : (bn == 80 ? launch_heads<80>(ahi, alo, whi, wlo, a, st) : launch_heads<64>(ahi, alo, whi, wlo, a, st));
   if (rc) return rc;
   simdr_heads_finalize_kernel<<<1, 1024, 0, st>>>((const double*)workspace, (N + bn - 1) / bn, weight, B, K, Lx, Ly, loss);
-  return check_launch();
+  rc = check_launch();
+  if (rc == LHN_OK) {
+    const int stages = bn == 128 ? HeadsTile<128>::kStages : (bn == 80 ? HeadsTile<80>::kStages : HeadsTile<64>::kStages);
+    simdr_record(5, 1, LHN_BF16, 8, stages, (int64_t)((N + bn - 1) / bn) * ((M + kHeadsBM - 1) / kHeadsBM), 1, 1, bn);
+  }
+  return rc;
 }

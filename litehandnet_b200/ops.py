@@ -635,9 +635,10 @@ def render_simdr(joints, vis, image_size, k=2, sigma=2):
     Lx, Ly = int(image_size[0] * k), int(image_size[1] * k)
     sx = torch.empty((B, K, Lx), dtype=torch.float32, device=joints.device)
     sy = torch.empty((B, K, Ly), dtype=torch.float32, device=joints.device)
-    rc = L.lib().lhn_render_simdr(L.ptr(joints), joints.shape[2], L.ptr(vis), vis.shape[2], B, K, Lx, Ly,
-                                  float(k), float(sigma), L.ptr(sx), L.ptr(sy), L.stream())
-    L.check(rc, "lhn_render_simdr")
+    # sigma as a double: the reference's denominator 2 * sigma ** 2 is formed in f64 and rounded to f32 once
+    rc = L.lib().lhn_render_simdr_f64sigma(L.ptr(joints), joints.shape[2], L.ptr(vis), vis.shape[2], B, K, Lx, Ly,
+                                           float(k), float(sigma), L.ptr(sx), L.ptr(sy), L.stream())
+    L.check(rc, "lhn_render_simdr_f64sigma")
     return sx, sy
 
 

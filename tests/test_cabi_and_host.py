@@ -129,6 +129,45 @@ def test_k1_launch_record_without_gpu(lib_path):
     assert seen == [(0, 0, 0), (-3, 0, 0)], seen
 
 
+def test_simdr_launch_record_without_gpu(lib_path):
+    """lhn_simdr_last_launch: a null pointer is refused; a fresh thread reads family == 0, and every SimDR entry point
+    clears the record on entry, so a call rejected before its launch leaves it cleared."""
+    import threading
+    from litehandnet_b200 import _lib
+    lib = _lib.lib()
+    assert ctypes.sizeof(_lib.SimdrLaunchInfo) == 9 * 4
+    assert lib.lhn_simdr_last_launch(None) == -1
+    p = ctypes.c_void_p(16)
+    rejected = {    # each call fails its argument checks before any device work
+        "render": lambda: lib.lhn_render_simdr(p, 3, p, 1, 1, 21, 512, 512, 2.0, 0.0, p, p, None),
+        "render_f64sigma": lambda: lib.lhn_render_simdr_f64sigma(p, 3, p, 1, 1, 21, 512, 512, 2.0, -1.0, p, p, None),
+        "decode": lambda: lib.lhn_decode_simdr_flags(p, p, _lib.F32, 1, 0, 512, 512, 2, None, None, 0, None, p, None, 0,
+                                                     None),
+        "loss": lambda: lib.lhn_simdr_smoothl1(p, p, p, p, p, _lib.F32, 1, 21, 512, 512, p, 8, p, None),
+        "backward": lambda: lib.lhn_simdr_smoothl1_backward(p, p, p, p, p, _lib.F32, 1, 21, 512, 512, 1.0, None, p, 4,
+                                                           p, p, None),
+        "heads": lambda: lib.lhn_simdr_heads_loss(p, p, p, p, p, p, p, p, 1, 21, 100, 512, 512, p, 1 << 20, p, None,
+                                                  None, None),
+        "heads_f32": lambda: lib.lhn_simdr_heads_loss_f32(p, p, p, p, p, p, p, 1, 21, 4096, 512, 512, p, 0, p, None,
+                                                          None, None),
+    }
+    seen = []
+
+    def probe():
+        r = _lib.SimdrLaunchInfo()
+        r.family, r.ctas = 7, 7
+        seen.append(("fresh", lib.lhn_simdr_last_launch(ctypes.byref(r)), r.family, r.ctas))
+        for name, call in rejected.items():
+            rc = call()
+            r.family = 7
+            seen.append((name, rc < 0, lib.lhn_simdr_last_launch(ctypes.byref(r)), r.family))
+
+    t = threading.Thread(target=probe)
+    t.start()
+    t.join()
+    assert seen == [("fresh", 0, 0, 0)] + [(n, True, 0, 0) for n in rejected], seen
+
+
 def test_no_cpu_fallback():
     """CPU tensors are refused loudly; nothing under litehandnet_b200/ imports the oracle."""
     from litehandnet_b200 import _lib, ops

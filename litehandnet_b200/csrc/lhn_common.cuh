@@ -143,6 +143,13 @@ __device__ __forceinline__ float warp_sum(float v) {
   return v;
 }
 
+// One joint's term of the fixed-point EPE sum (epe_fix counters): the f32 distance in 2^-20 px, rounded to nearest
+// (a power of two, so d * 2^20 is exact).  A distance that is NaN, infinite or too large for the int64 term
+// (d >= 2^43 px) adds nothing, and the joint still counts in epe_valid.  Every producer of the counters uses this.
+__device__ __forceinline__ unsigned long long epe_fix_term(float d) {
+  return d < 0x1p43f ? (unsigned long long)__float2ll_rn(d * 1048576.f) : 0ull;
+}
+
 // ---------------------------------------------------------------------------------------------
 // Gaussian target geometry (generateTarget.py:100-154 MSRA, :162-243 UDP), shared by the fused kernel,
 // the CTA-per-plane fallback, lhn_render_targets, the two-pass backward and the one-pass loss + gradient so

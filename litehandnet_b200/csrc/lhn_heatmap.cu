@@ -405,7 +405,7 @@ __global__ void __launch_bounds__(NT) heatmap_plane_kernel(const __grid_constant
         float d = (float)sqrt(__dadd_rn(__dmul_rn(ddx, ddx), __dmul_rn(ddy, ddy)));
         unsigned long long* epe = cnt + (int64_t)(3 + a.auc_steps) * K;
         atomicAdd(epe + k, 1ull);
-        atomicAdd(epe + K + k, (unsigned long long)llrint((double)d * 1048576.0));
+        atomicAdd(epe + K + k, epe_fix_term(d));
       }
     }
   }

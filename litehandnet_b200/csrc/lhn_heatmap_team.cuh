@@ -684,7 +684,7 @@ heatmap_team_kernel(const __grid_constant__ HmArgs a) {
           } else if (lane == 2) {
             unsigned long long* epe = cta_cnt + (int64_t)(3 + a.auc_steps) * Ki;
             bump(epe + k);
-            atomicAdd(epe + Ki + k, (unsigned long long)llrint((double)d * 1048576.0));
+            atomicAdd(epe + Ki + k, epe_fix_term(d));
           }
         }
       }

@@ -1,6 +1,7 @@
 // K3 — PCK / AUC / EPE accumulation as shardable integer counters, and the legacy evaluate_pck.
-// The arithmetic of _calc_distances is reproduced in the dtype numpy would promote to (f64 unless
-// every input is f32), rounded to f32 and compared with the f32 threshold, so hit counts are
+// The arithmetic of _calc_distances is reproduced step by step in the dtype numpy would promote to (the
+// difference pred - gt in f32 when both are f32, the division and everything after it in f64 unless the
+// normaliser is f32 too), rounded to f32 and compared with the f32 threshold, so hit counts are
 // bit-exact; counters are int64 and order-independent, hence identical for any sharding.
 #include <cstdlib>
 #include <math_constants.h>
@@ -21,6 +22,7 @@ struct PckArgs {
   int64_t N; int K, T;
   float thr[kMaxThr];
   int all_f32;
+  int diff_f32;               // pred and gt are both f32: numpy takes their difference in f32
   int sorted_thr;             // thr[] is non-decreasing (host-checked): histogram counting
   unsigned long long* counters;
 };
@@ -47,10 +49,12 @@ __global__ void __launch_bounds__(256) pck_accumulate_kernel(const __grid_consta
   for (int i = threadIdx.x; i < ncnt; i += blockDim.x) sc[i] = 0ull;
   for (int i = threadIdx.x; i < (T + 1) * K; i += blockDim.x) hist[i] = 0u;
   __syncthreads();
-  const int64_t total = a.N * K;
   const int64_t nthreads = (int64_t)gridDim.x * blockDim.x;
-  const int64_t stride = (nthreads + K - 1) / K * K;                 // a multiple of K: k is loop-invariant
+  // the stride is rounded DOWN to a multiple of K, so k is loop-invariant and the threads at e0 >= stride (fewer than K)
+  // take no element: every element is visited exactly once.  Uncapped grids have nthreads >= N*K, hence stride >= N*K.
+  const int64_t stride = nthreads / K * K;
   const int64_t e0 = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  const int64_t total = e0 < stride ? a.N * K : 0;
   const int k = (int)(e0 % K);
   const int64_t n_step = stride / K;
   int64_t n = e0 / K;
@@ -60,7 +64,7 @@ __global__ void __launch_bounds__(256) pck_accumulate_kernel(const __grid_consta
   const float thr0 = T > 0 ? a.thr[0] : 0.f;
   auto consume = [&](float d) {
     ++valid;
-    if (d == d) dsum += (unsigned long long)__float2ll_rn(d * 1048576.f);   // a power of two: exact in f32 as in f64
+    dsum += epe_fix_term(d);                           // NaN, inf and d >= 2^43 add nothing
     if (T == 1) {
       hit1 += (d < thr0) ? 1u : 0u;
     } else if (a.sorted_thr) {
@@ -123,7 +127,11 @@ __global__ void __launch_bounds__(256) pck_accumulate_kernel(const __grid_consta
       const double gx = ld_as_f64(a.gt, a.gt_dtype, e * a.gt_stride);
       const double gy = ld_as_f64(a.gt, a.gt_dtype, e * a.gt_stride + 1);
       const double dx = nx < 0.0 ? 1e6 : nx, dy = ny < 0.0 ? 1e6 : ny;
-      const double qx = __ddiv_rn(__dsub_rn(px, gx), dx), qy = __ddiv_rn(__dsub_rn(py, gy), dy);
+      // `preds - targets` comes first in numpy: two f32 arrays subtract in f32, and only the division by an f64
+      // normaliser (or the python-float constant) promotes
+      const double ex = a.diff_f32 ? (double)__fsub_rn((float)px, (float)gx) : __dsub_rn(px, gx);
+      const double ey = a.diff_f32 ? (double)__fsub_rn((float)py, (float)gy) : __dsub_rn(py, gy);
+      const double qx = __ddiv_rn(ex, dx), qy = __ddiv_rn(ey, dy);
       d = (float)__dsqrt_rn(__dadd_rn(__dmul_rn(qx, qx), __dmul_rn(qy, qy)));
     }
     if (!m || nx == 0.0 || ny == 0.0) continue;        // masked joint / _mask[normalize == 0 rows] = False
@@ -242,7 +250,8 @@ extern "C" int lhn_pck_accumulate(const void* pred, int pred_dtype, int pred_str
                                   const void* normalize, int norm_dtype, double norm_const, int64_t N,
                                   int K, const float* thr, int T, int64_t* counters,
                                   lhn_stream_t stream) {
-  if (!pred || !gt || !mask || !counters || N < 0 || K <= 0 || T < 0 || T > kMaxThr ||
+  // an empty shard (N == 0) reads no element: its arrays may be null, as torch's empty CUDA tensors are
+  if ((N > 0 && (!pred || !gt || !mask)) || !counters || N < 0 || K <= 0 || T < 0 || T > kMaxThr ||
       pred_stride < 2 || gt_stride < 2 || (T > 0 && !thr))
     return LHN_EINVAL;
   auto okdt = [](int d) { return d == LHN_F32 || d == LHN_F64; };
@@ -257,6 +266,7 @@ extern "C" int lhn_pck_accumulate(const void* pred, int pred_dtype, int pred_str
   for (int i = 0; i < T; ++i) { a.thr[i] = thr[i]; if (i > 0 && !(thr[i] >= thr[i - 1])) a.sorted_thr = 0; }
   // numpy promotion: f32 only if every array operand is f32 (a python-float constant is f64)
   a.all_f32 = pred_dtype == LHN_F32 && gt_dtype == LHN_F32 && normalize && norm_dtype == LHN_F32;
+  a.diff_f32 = pred_dtype == LHN_F32 && gt_dtype == LHN_F32;
   a.counters = reinterpret_cast<unsigned long long*>(counters);
   const int threads = 256;
   int64_t need = (N * K + threads - 1) / threads, cap = (int64_t)num_sms() * 8;

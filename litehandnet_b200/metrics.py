@@ -63,7 +63,9 @@ def keypoint_auc(pred, gt, mask, normalize, num_step=20):
 
 def keypoint_epe(pred, gt, mask):
     """Mean end-point error over the visible joints.  The distances are summed in 2^-20 px fixed point
-    (int64: exact, order-independent, shardable); the reference sums f32 distances."""
+    (int64: exact, order-independent, shardable); the reference sums f32 distances.  A distance that is NaN,
+    infinite or at least 2^43 px (a NaN or inf prediction, say) cannot be held in that sum: it adds nothing and the
+    joint still counts, where the reference would return NaN or inf."""
     K = pred.shape[1]
     n = pred.shape[0]
     dev_pred, _ = _up(pred)
@@ -228,14 +230,24 @@ def mpii_evaluate(results, gt_dict, metric='PCKh'):
     keep = torch.ones_like(ids_s, dtype=torch.bool)
     keep[1:] = ids_s[1:] != ids_s[:-1]
     preds = preds[order][keep].contiguous()
-    rng = np.arange(0, 0.5 + 0.01, 0.01)
-    thr = [0.5] + [float(t) for t in rng]
+    thr = MPII_THRESHOLDS
     K = preds.shape[1]
-    c = mpii_pckh_counters(preds, gt_dict, thr).cpu().numpy().reshape(len(thr) + 1, K).astype(np.float64)
+    c = mpii_pckh_counters(preds, gt_dict, thr).cpu().numpy().reshape(len(thr) + 1, K)
+    return mpii_table(c, gt_dict['dataset_joints'])
+
+
+# PCKh@0.5, then the rows of pckAll (np.arange(0, 0.5 + 0.01, 0.01)) in the reference's evaluate
+MPII_THRESHOLDS = [0.5] + [float(t) for t in np.arange(0, 0.5 + 0.01, 0.01)]
+
+
+def mpii_table(counters, dataset_joints):
+    """The name/value table of TopDownMpiiDataset.evaluate from the counters [len(MPII_THRESHOLDS) + 1, K]
+    (hits per threshold, then the joint count) of mpii_pckh_counters."""
+    c = np.asarray(counters).astype(np.float64)
     jnt_count = c[-1]
     PCKh = 100. * c[0] / jnt_count
     pck10 = (100. * c[1 + 10] / jnt_count).astype(np.float32)                  # pckAll is a float32 table
-    names = np.asarray(gt_dict['dataset_joints'])
+    names = np.asarray(dataset_joints)
     J = {n: np.where(names == n)[1][0] for n in ('head', 'lsho', 'lelb', 'lwri', 'lhip', 'lkne', 'lank', 'rsho',
                                                  'relb', 'rwri', 'rkne', 'rank', 'rhip')}
     PCKh = np.ma.array(PCKh, mask=False); PCKh.mask[6:8] = True

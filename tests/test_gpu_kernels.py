@@ -506,23 +506,29 @@ def test_pck_counters_golden(ops, L):
 
 
 def test_pck_counters_sharded_equal_monolithic(ops, L):
-    N, K = 4096, 16
-    hm, cen = synth.blob_heatmaps(8, K, 64, 64, seed=71)
-    rng = np.random.default_rng(72)
-    pred = rng.uniform(0, 256, (N, K, 2)).astype(np.float32)
-    gt = (pred + rng.normal(0, 12, (N, K, 2))).astype(np.float32)
-    mask = rng.uniform(0, 1, (N, K)) < 0.9
-    nor = np.repeat(rng.uniform(60, 200, (N, 1)), 2, 1)
-    thr = [0.05, 0.1, 0.2, 0.5]
-    mono = nump(ops.pck_accumulate(cu(pred.astype(np.float64)), cu(gt), cu(mask), thr, normalize=cu(nor)))
-    sharded = torch.zeros((len(thr) + 2) * K, dtype=torch.int64, device=DEV)
-    for sh in np.array_split(np.arange(N), 8):
-        ops.pck_accumulate(cu(pred[sh].astype(np.float64)), cu(gt[sh]), cu(mask[sh]), thr, normalize=cu(nor[sh]),
-                           counters=sharded)
-    assert np.array_equal(mono, nump(sharded))
-    hits, valid = O.pck_counters(pred.astype(np.float64), gt, mask, thr, nor)
-    assert np.array_equal(mono.reshape(len(thr) + 2, K)[:len(thr)], hits)
-    assert np.array_equal(mono.reshape(len(thr) + 2, K)[len(thr)], valid)
+    """Eight even shards of 4096 x 16, and uneven shards of 21-joint samples past the capped grid (8 * SMs blocks of
+    256 threads), one shard past it by itself, with the cap not a multiple of 21: the grid stride must still visit
+    every element once."""
+    cap = 8 * torch.cuda.get_device_properties(0).multi_processor_count * 256
+    S = cap // 21
+    assert cap % 21 and (S + 3) * 21 > cap
+    for N, K, bounds in ((4096, 16, [int(s[0]) for s in np.array_split(np.arange(4096), 8)] + [4096]),
+                         (2 * S + 5, 21, [0, 7, S + 10, 2 * S + 4, 2 * S + 5])):
+        rng = np.random.default_rng(72)
+        pred = rng.uniform(0, 256, (N, K, 2)).astype(np.float32)
+        gt = (pred + rng.normal(0, 12, (N, K, 2))).astype(np.float32)
+        mask = rng.uniform(0, 1, (N, K)) < 0.9
+        nor = np.repeat(rng.uniform(60, 200, (N, 1)), 2, 1)
+        thr = [0.05, 0.1, 0.2, 0.5]
+        mono = nump(ops.pck_accumulate(cu(pred.astype(np.float64)), cu(gt), cu(mask), thr, normalize=cu(nor)))
+        sharded = torch.zeros((len(thr) + 2) * K, dtype=torch.int64, device=DEV)
+        for a, b in zip(bounds[:-1], bounds[1:]):
+            ops.pck_accumulate(cu(pred[a:b].astype(np.float64)), cu(gt[a:b]), cu(mask[a:b]), thr,
+                               normalize=cu(nor[a:b]), counters=sharded)
+        assert np.array_equal(mono, nump(sharded)), (N, K)
+        hits, valid = O.pck_counters(pred.astype(np.float64), gt, mask, thr, nor)
+        assert np.array_equal(mono.reshape(len(thr) + 2, K)[:len(thr)], hits), (N, K)
+        assert np.array_equal(mono.reshape(len(thr) + 2, K)[len(thr)], valid), (N, K)
 
 
 def test_fused_decode_pck_counters(ops, L):

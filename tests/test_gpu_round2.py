@@ -12,16 +12,35 @@ pytestmark = pytest.mark.gpu
 DEV = "cuda"
 
 
-@pytest.mark.parametrize("K,N,mask_prob", [(16, 512, 0.9), (21, 300, 0.5), (7, 40, 0.9), (16, 64, 0.0)])
-def test_metrics_finalize_equals_host_expressions(K, N, mask_prob):
+def _fin(K, N, mask_prob, T=20, dead=(), first=False):
+    # the first four cases keep the ids they had before T and `dead` were parameters
+    return pytest.param(K, N, mask_prob, T, dead, id=f"{K}-{N}-{mask_prob}" + ("" if first else f"-T{T}-dead{len(dead)}"))
+
+
+# np.mean's pairwise sum changes form at 8 averaged joints (eight accumulators, then a tail) and ends at 128; joints
+# without a valid sample (`dead`) are left out of the mean, so they move the count across those edges
+FINALIZE_CASES = [
+    _fin(16, 512, 0.9, first=True), _fin(21, 300, 0.5, first=True), _fin(7, 40, 0.9, dead=(3,), first=True),
+    _fin(16, 64, 0.0, first=True),
+    _fin(1, 64, 0.9), _fin(8, 64, 0.9), _fin(9, 64, 0.9), _fin(9, 64, 0.9, dead=(4,)), _fin(15, 64, 0.9),
+    _fin(16, 64, 0.9, T=1, dead=(0,)), _fin(17, 64, 0.9), _fin(17, 64, 0.9, dead=(16,)), _fin(17, 64, 0.9, T=0, dead=(1, 2)),
+    _fin(64, 32, 0.9, T=64), _fin(64, 32, 0.9, dead=tuple(range(55))), _fin(127, 16, 0.9), _fin(128, 16, 0.9),
+    _fin(128, 16, 0.9, T=1, dead=tuple(range(0, 128, 2))), _fin(128, 16, 0.9, dead=tuple(range(121))),
+    _fin(128, 8, 0.0, T=64),
+]
+
+
+@pytest.mark.parametrize("K,N,mask_prob,T,dead", FINALIZE_CASES)
+def test_metrics_finalize_equals_host_expressions(K, N, mask_prob, T, dead):
     """lhn_metrics_finalize (device) == _report_metric's NumPy expressions on the same counters, bit for bit
-    (datasets/base_dataset.py:193-261, top_down_eval.py:44-62,167-196), and == the oracle on the decoded points."""
+    (datasets/base_dataset.py:193-261, top_down_eval.py:44-62,167-196), and == the oracle on the decoded points.
+    K from 1 to 128, T = 0, 1, 20 and 64 AUC steps, all-zero counters."""
     hm, cen = synth.blob_heatmaps(N, K, 64, 64, seed=11, device=DEV)
     c, s = synth.bbox_center_scale(N, seed=12, device=DEV)
     gt, mask, wh = synth.pck_inputs(cen, seed=13, device=DEV, mask_prob=mask_prob)
-    if K == 7:
-        mask[:, 3] = False                                  # a joint without any valid sample: acc = -1, left out of the mean
-    acc = M.MetricAccumulator(K, device=DEV)
+    for k in dead:
+        mask[:, k] = False                                  # a joint without any valid sample: acc = -1, left out of the mean
+    acc = M.MetricAccumulator(K, device=DEV, auc_steps=T)
     r = acc.update_from_heatmaps(hm, c, s, gt, mask, wh, post_process="default")
     host = acc.compute()
     dev = acc.compute(on_device=True)
@@ -36,8 +55,13 @@ def test_metrics_finalize_equals_host_expressions(K, N, mask_prob):
         t = wh.max(1).values.double().cpu().numpy()
         _, pck, _ = O.keypoint_pck_accuracy(p64, gt.cpu().numpy(), mask.cpu().numpy(), 0.2, np.stack([t, t], 1))
         np.testing.assert_allclose(dev["PCK"], pck, rtol=1e-12)
-        np.testing.assert_allclose(dev["AUC"], O.keypoint_auc(p64, gt.cpu().numpy(), mask.cpu().numpy(), 30), rtol=1e-12)
+        if T:
+            np.testing.assert_allclose(dev["AUC"], O.keypoint_auc(p64, gt.cpu().numpy(), mask.cpu().numpy(), 30, T),
+                                       rtol=1e-12)
+        n_avg = int((cnt[1] > 0).sum())
+        assert n_avg == K - len(dead)                         # the number of averaged joints the case aims at
     else:
+        assert not cnt.any()
         assert dev["PCK"] == 0 and dev["AUC"] == 0 and dev["EPE"] == 0
 
 
@@ -47,6 +71,8 @@ def test_metrics_finalize_rejects_bad_arguments():
         ops.metrics_finalize(cnt, 15)
     with pytest.raises(L.LhnError):
         ops.metrics_finalize(cnt.int(), 16)
+    with pytest.raises(L.LhnError):                         # past numpy's 128-element pairwise block
+        ops.metrics_finalize(torch.zeros(25 * 129, dtype=torch.int64, device=DEV), 129)
 
 
 # ---- SimDRLoss heads fused into one tcgen05 kernel (centernet_simdr_loss.py:42-69) ---------------------------

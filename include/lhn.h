@@ -439,6 +439,43 @@ LHN_API int lhn_loss_mse_multi(int n_tensors, const void* const* outputs, const 
                                double* sums, float* per_tensor_loss, float* loss, int accumulate,
                                lhn_stream_t stream);
 
+/* ---- the multi-scale loss with every scale's target rendered in-kernel ---------------------------------------------
+ * SRHandNetLoss._forward_only_heatmap (loss/loss.py:59-66) from the joints: loss = scale * sum_i loss_weight_i *
+ * f32(L_i), L_i = DistanceLoss / JointsDistanceLoss (heatmapLoss.py:195-265) of scale i's output against the target
+ * lhn_render_targets would draw for it (rp->unbiased, rp->pos_value, rp->loss_mode and rp->image_w / image_h shared;
+ * the scale's own H, W, sigma and feature stride; target_weight after the visibility rule of ITS plane size).  The
+ * targets are never materialised.  All scales share joints f32 [B, K, joints_stride] and vis f32 [B, K, vis_stride]
+ * (column 0); rp->num_stacks and rp->sigma are not read.  `scales` is a HOST array of n_scales <=
+ * LHN_LOSS_MAX_TENSORS descriptors. */
+typedef struct {
+  const void* output;      /* [B, K, H, W] of `dtype`, planes contiguous, element strides stride_b / stride_c */
+  void* grad;              /* backward: contiguous [B, K, H, W] of `dtype`, or NULL to skip this scale; forward: unused */
+  float* out_weight;       /* forward: f32 [B*K] target_weight of this scale, or NULL; backward: unused */
+  int64_t stride_b, stride_c;
+  int32_t H, W;
+  float sigma;
+  float loss_weight;       /* forward: the weight of this scale's term; backward: its gradient's scale */
+} lhn_loss_scale;
+
+/* Forward, ONE launch: the grid dealing, fixed-order two-level reduction and last-CTA finalise of
+ * lhn_loss_mse_multi (bitwise reproducible for a given shape and device).  sums (optional) f64 [n_scales, 4] =
+ * (S_pos, S_neg, N_pos, numel) per scale, which the backward needs; per_scale_loss (optional) f32 [n_scales] = L_i;
+ * loss (optional) f32 [1].  workspace: lhn_render_loss_multi_workspace_bytes() bytes, 16-byte aligned, zeroed once
+ * and left zero (the same size and contract as lhn_loss_mse_multi's, so one buffer may serve both on one stream). */
+LHN_API int64_t lhn_render_loss_multi_workspace_bytes(void);
+LHN_API int lhn_render_loss_multi(int n_scales, const lhn_loss_scale* scales, int dtype, int64_t B, int K,
+                                  const lhn_render_params* rp, const float* joints, int joints_stride,
+                                  const float* vis, int vis_stride, int sum_reduction, float scale,
+                                  void* workspace, int64_t workspace_bytes, double* sums, float* per_scale_loss,
+                                  float* loss, lhn_stream_t stream);
+/* Backward, ONE launch writing every scale's gradient (scales with grad == NULL are skipped): bit for bit
+ * lhn_render_loss_backward on scale i with sums + 4 i and scale = loss_weight_i, for an upstream gradient
+ * grad_out[0] (f32 [1] device pointer, NULL = 1). */
+LHN_API int lhn_render_loss_backward_multi(int n_scales, const lhn_loss_scale* scales, int dtype, int64_t B, int K,
+                                           const lhn_render_params* rp, const float* joints, int joints_stride,
+                                           const float* vis, int vis_stride, const double* sums, int sum_reduction,
+                                           const float* grad_out, lhn_stream_t stream);
+
 /* ---- SimDRLoss with its two nn.Linear heads fused (centernet_simdr_loss.py:42-69) -------------------------------
  * pred_x | pred_y = heatmap.flatten(2) @ [Wx ; Wy]^T + [bx ; by], then KLDiscretLoss (:27-39) — ONE tcgen05 kernel:
  * the predictions stay in tensor memory, the epilogue takes SmoothL1 against the targets and row-reduces it; a

@@ -45,6 +45,7 @@ EXPORTS = [
     "lhn_simdr_smoothl1_backward", "lhn_mpii_pckh_accumulate", "lhn_region_bbox_decode", "lhn_heatmap_nms",
     "lhn_vector_nms", "lhn_refine_points", "lhn_decode_heatmap_roi", "lhn_box_nms", "lhn_render_region_wh", "lhn_dark_refine_points",
     "lhn_k1_last_launch", "lhn_simdr_last_launch",
+    "lhn_render_loss_multi_workspace_bytes", "lhn_render_loss_multi", "lhn_render_loss_backward_multi",
 ]
 
 
@@ -58,6 +59,13 @@ class RenderParams(C.Structure):
     _fields_ = [("loss_mode", C.c_int32), ("unbiased", C.c_int32), ("num_stacks", C.c_int32),
                 ("reserved", C.c_int32), ("image_w", C.c_float), ("image_h", C.c_float),
                 ("pos_value", C.c_float), ("sigma", C.c_float * MAX_STACKS)]
+
+
+class LossScale(C.Structure):
+    """lhn_loss_scale: one scale of lhn_render_loss_multi / lhn_render_loss_backward_multi."""
+    _fields_ = [("output", C.c_void_p), ("grad", C.c_void_p), ("out_weight", C.c_void_p), ("stride_b", C.c_int64),
+                ("stride_c", C.c_int64), ("H", C.c_int32), ("W", C.c_int32), ("sigma", C.c_float),
+                ("loss_weight", C.c_float)]
 
 
 class Exchange(C.Structure):
@@ -139,6 +147,12 @@ def _declare(lib):
     lib.lhn_loss_mse_workspace_bytes.restype = i64
     lib.lhn_loss_mse_multi.argtypes = [i32, C.POINTER(vp), C.POINTER(vp), C.POINTER(vp), C.POINTER(i64), C.POINTER(i64),
                                        C.POINTER(f32), i32, i32, f32, i32, f32, vp, i64, vp, vp, vp, i32, vp]
+    lib.lhn_render_loss_multi_workspace_bytes.argtypes = []
+    lib.lhn_render_loss_multi_workspace_bytes.restype = i64
+    lib.lhn_render_loss_multi.argtypes = [i32, C.POINTER(LossScale), i32, i64, i32, C.POINTER(RenderParams), vp, i32,
+                                          vp, i32, i32, f32, vp, i64, vp, vp, vp, vp]
+    lib.lhn_render_loss_backward_multi.argtypes = [i32, C.POINTER(LossScale), i32, i64, i32, C.POINTER(RenderParams),
+                                                   vp, i32, vp, i32, vp, i32, vp, vp]
     lib.lhn_loss_finalize.argtypes = [vp, i32, i32, f32, vp, i32, vp]
     lib.lhn_render_targets.argtypes = [vp, i32, vp, i32, i64, i32, i32, i32, C.POINTER(RenderParams),
                                        vp, vp, vp]

@@ -70,6 +70,37 @@ struct RenderBwdArgs {
   const double* sums; const float* grad_out;
 };
 
+// One plane of the rendered-target gradient, strided over threads t0, t0 + nt, ...: the per-element arithmetic that
+// lhn_render_loss_backward and lhn_render_loss_backward_multi share, so the two write the same bits.
+template <typename T>
+__device__ __forceinline__ void render_grad_plane(const T* src, T* dst, const float* ex, const float* ey, int W, int H,
+                                                  float wp, float wn, bool bal, float pos_value, int t0, int nt) {
+  const bool vec = (W & 3) == 0 && (reinterpret_cast<uintptr_t>(src) % (4 * sizeof(T)) == 0) &&
+                   (reinterpret_cast<uintptr_t>(dst) % (4 * sizeof(T)) == 0);
+  if (vec) {
+    const int QR = W >> 2, nq = (H * W) >> 2;
+    for (int q = t0; q < nq; q += nt) {
+      const int row = q / QR, cq = q - row * QR;
+      const float4 gx = *reinterpret_cast<const float4*>(ex + 4 * cq);
+      const float gy = ey[row];
+      const float4 o = ldg_stream4<T>(src + 4 * q);
+      const float g0 = gx.x * gy, g1 = gx.y * gy, g2 = gx.z * gy, g3 = gx.w * gy;
+      float4 r;
+      r.x = ((bal && g0 > pos_value) ? wp : wn) * fmaf(-gx.x, gy, o.x);
+      r.y = ((bal && g1 > pos_value) ? wp : wn) * fmaf(-gx.y, gy, o.y);
+      r.z = ((bal && g2 > pos_value) ? wp : wn) * fmaf(-gx.z, gy, o.z);
+      r.w = ((bal && g3 > pos_value) ? wp : wn) * fmaf(-gx.w, gy, o.w);
+      Store4<T>::st(dst + 4 * q, r);
+    }
+  } else {
+    for (int e = t0; e < H * W; e += nt) {
+      const int y = e / W, x = e - y * W;
+      const float g = ex[x] * ey[y];
+      dst[e] = Store4<T>::from(((bal && g > pos_value) ? wp : wn) * fmaf(-ex[x], ey[y], Elem<T>::to_f32(src[e])));
+    }
+  }
+}
+
 template <typename T>
 __global__ void __launch_bounds__(128) render_loss_backward_kernel(const __grid_constant__ RenderBwdArgs a) {
   extern __shared__ float tab[];   // ex[W], ey[H]
@@ -90,35 +121,69 @@ __global__ void __launch_bounds__(128) render_loss_backward_kernel(const __grid_
   float cpos, cneg;
   loss_coefs(a.sums, a.loss_mode, a.sum_reduction, a.scale, a.grad_out, cpos, cneg);
   if (a.loss_mode == LHN_LOSS_JOINTS_MSE) w *= w;
-  const float wp = w * cpos, wn = w * cneg;
-  const bool bal = a.loss_mode == LHN_LOSS_DISTANCE_BALANCE;
   __syncthreads();
   const T* src = reinterpret_cast<const T*>(a.hm) + b * a.stride_b + (int64_t)c * a.stride_c;
   T* dst = reinterpret_cast<T*>(a.grad) + p * (int64_t)H * W;
-  const bool vec = (W & 3) == 0 && (reinterpret_cast<uintptr_t>(src) % (4 * sizeof(T)) == 0) &&
-                   (reinterpret_cast<uintptr_t>(dst) % (4 * sizeof(T)) == 0);
-  if (vec) {
-    const int QR = W >> 2, nq = (H * W) >> 2;
-    for (int q = threadIdx.x; q < nq; q += blockDim.x) {
-      const int row = q / QR, cq = q - row * QR;
-      const float4 gx = *reinterpret_cast<const float4*>(ex + 4 * cq);
-      const float gy = ey[row];
-      const float4 o = ldg_stream4<T>(src + 4 * q);
-      const float g0 = gx.x * gy, g1 = gx.y * gy, g2 = gx.z * gy, g3 = gx.w * gy;
-      float4 r;
-      r.x = ((bal && g0 > a.pos_value) ? wp : wn) * fmaf(-gx.x, gy, o.x);
-      r.y = ((bal && g1 > a.pos_value) ? wp : wn) * fmaf(-gx.y, gy, o.y);
-      r.z = ((bal && g2 > a.pos_value) ? wp : wn) * fmaf(-gx.z, gy, o.z);
-      r.w = ((bal && g3 > a.pos_value) ? wp : wn) * fmaf(-gx.w, gy, o.w);
-      Store4<T>::st(dst + 4 * q, r);
-    }
-  } else {
-    for (int e = threadIdx.x; e < H * W; e += blockDim.x) {
-      const int y = e / W, x = e - y * W;
-      const float g = ex[x] * ey[y];
-      dst[e] = Store4<T>::from(((bal && g > a.pos_value) ? wp : wn) * fmaf(-ex[x], ey[y], Elem<T>::to_f32(src[e])));
-    }
-  }
+  render_grad_plane<T>(src, dst, ex, ey, W, H, w * cpos, w * cneg, a.loss_mode == LHN_LOSS_DISTANCE_BALANCE,
+                       a.pos_value, threadIdx.x, blockDim.x);
+}
+
+// ---- every scale of SRHandNetLoss in one launch (loss/loss.py:59-66): one WARP per plane ----------------
+// Scale i's planes are warps [i * B * K, (i + 1) * B * K) of the grid.  A warp renders its plane's ex[W], ey[H]
+// into warp-private shared memory and writes the gradient with render_grad_plane; the coefficient comes from the
+// scale's own row of the forward's sums and its loss weight.  A 16 x 16 plane is 64 quads, two per lane: a
+// 128-thread CTA per plane would leave half its threads without work.
+constexpr int kBwdMultiWarps = 8;
+
+struct RenderBwdScale {
+  const void* hm; void* grad;
+  int64_t stride_b, stride_c;
+  double feat_x, feat_y;
+  float sigma, scale;
+  int H, W, sums_row;
+};
+
+struct RenderBwdMultiArgs {
+  RenderBwdScale s[LHN_LOSS_MAX_TENSORS];
+  int n, K;
+  int64_t BK;
+  const float* joints; int joints_stride;
+  const float* vis; int vis_stride;
+  int unbiased, loss_mode, sum_reduction, tab_stride;
+  float pos_value;
+  const double* sums; const float* grad_out;
+};
+
+template <typename T>
+__global__ void __launch_bounds__(kBwdMultiWarps * 32) render_loss_backward_multi_kernel(
+    const __grid_constant__ RenderBwdMultiArgs a) {
+  extern __shared__ float4 btab4[];
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const int64_t gw = (int64_t)blockIdx.x * kBwdMultiWarps + warp;
+  if (gw >= a.n * a.BK) return;
+  const int i = (int)(gw / a.BK);
+  const int64_t p = gw - i * a.BK;
+  const RenderBwdScale& s = a.s[i];
+  const int W = s.W, H = s.H;
+  float* ex = reinterpret_cast<float*>(btab4) + warp * a.tab_stride;
+  float* ey = ex + W;
+  const int64_t b = p / a.K;
+  const int k = (int)(p - b * a.K);
+  const float* jp = a.joints + p * (int64_t)a.joints_stride;
+  const double sig = (double)s.sigma;
+  const RenderGeom g = render_geom(jp[0], jp[1], a.vis[p * (int64_t)a.vis_stride], sig, a.unbiased, s.feat_x,
+                                   s.feat_y, 0, 0.0, 0.0, W, H);
+  float w = g.w;
+  const double inv2s2 = 1.0 / (2.0 * sig * sig);
+  for (int e = lane; e < W + H; e += 32) ex[e] = table_entry(g, e, W, a.unbiased, inv2s2);
+  float cpos, cneg;
+  loss_coefs(a.sums + 4 * s.sums_row, a.loss_mode, a.sum_reduction, s.scale, a.grad_out, cpos, cneg);
+  if (a.loss_mode == LHN_LOSS_JOINTS_MSE) w *= w;
+  __syncwarp();
+  const T* src = reinterpret_cast<const T*>(s.hm) + b * s.stride_b + (int64_t)k * s.stride_c;
+  T* dst = reinterpret_cast<T*>(s.grad) + p * (int64_t)H * W;
+  render_grad_plane<T>(src, dst, ex, ey, W, H, w * cpos, w * cneg, a.loss_mode == LHN_LOSS_DISTANCE_BALANCE,
+                       a.pos_value, lane, 32);
 }
 
 // ---- KLDiscretLoss backward (centernet_simdr_loss.py:27-39): SmoothL1'(d) * mean_b(w)[j] / (K B L) ------
@@ -242,6 +307,49 @@ extern "C" int lhn_render_loss_backward(const void* hm, int dtype, int64_t B, in
     case LHN_BF16: render_loss_backward_kernel<__nv_bfloat16><<<(unsigned)a.n_planes, 128, smem, st>>>(a); break;
     case LHN_F16: render_loss_backward_kernel<__half><<<(unsigned)a.n_planes, 128, smem, st>>>(a); break;
     default: return LHN_EDTYPE;
+  }
+  return check_launch();
+}
+
+extern "C" int lhn_render_loss_backward_multi(int n_scales, const lhn_loss_scale* scales, int dtype, int64_t B,
+                                              int K, const lhn_render_params* rp, const float* joints,
+                                              int joints_stride, const float* vis, int vis_stride,
+                                              const double* sums, int sum_reduction, const float* grad_out,
+                                              lhn_stream_t stream) {
+  if (n_scales < 1 || n_scales > LHN_LOSS_MAX_TENSORS || !scales || !rp || !joints || !vis || !sums || B <= 0 ||
+      K <= 0 || joints_stride < 2 || vis_stride < 1)
+    return LHN_EINVAL;
+  if (dtype != LHN_F32 && dtype != LHN_BF16 && dtype != LHN_F16) return LHN_EDTYPE;
+  RenderBwdMultiArgs a{};
+  int tab = 0;
+  for (int i = 0; i < n_scales; ++i) {
+    const lhn_loss_scale& sc = scales[i];
+    double fx, fy;
+    if (!sc.output || scale_geometry(rp, sc.H, sc.W, sc.sigma, fx, fy) != LHN_OK) return LHN_EINVAL;
+    if (!sc.grad) continue;                               // this scale's gradient is not wanted
+    RenderBwdScale& s = a.s[a.n++];
+    s.hm = sc.output; s.grad = sc.grad; s.stride_b = sc.stride_b; s.stride_c = sc.stride_c;
+    s.feat_x = fx; s.feat_y = fy; s.sigma = sc.sigma; s.scale = sc.loss_weight; s.H = sc.H; s.W = sc.W;
+    s.sums_row = i;
+    if (sc.H + sc.W > tab) tab = sc.H + sc.W;
+  }
+  if (a.n == 0) return LHN_OK;
+  a.K = K; a.BK = B * K;
+  a.joints = joints; a.joints_stride = joints_stride; a.vis = vis; a.vis_stride = vis_stride;
+  a.unbiased = rp->unbiased; a.loss_mode = rp->loss_mode; a.sum_reduction = sum_reduction;
+  a.tab_stride = (tab + 3) & ~3; a.pos_value = rp->pos_value; a.sums = sums; a.grad_out = grad_out;
+  const int64_t blocks = (a.n * a.BK + kBwdMultiWarps - 1) / kBwdMultiWarps;
+  if (blocks > 0x7fffffffLL) return LHN_EINVAL;
+  const size_t smem = (size_t)kBwdMultiWarps * a.tab_stride * sizeof(float);
+  const void* fn = dtype == LHN_F32 ? (const void*)render_loss_backward_multi_kernel<float>
+                 : dtype == LHN_BF16 ? (const void*)render_loss_backward_multi_kernel<__nv_bfloat16>
+                                     : (const void*)render_loss_backward_multi_kernel<__half>;
+  if (set_dynamic_smem(fn, smem) != LHN_OK) return LHN_EINVAL;
+  cudaStream_t st = (cudaStream_t)stream;
+  switch (dtype) {
+    case LHN_F32: render_loss_backward_multi_kernel<float><<<(unsigned)blocks, kBwdMultiWarps * 32, smem, st>>>(a); break;
+    case LHN_BF16: render_loss_backward_multi_kernel<__nv_bfloat16><<<(unsigned)blocks, kBwdMultiWarps * 32, smem, st>>>(a); break;
+    default: render_loss_backward_multi_kernel<__half><<<(unsigned)blocks, kBwdMultiWarps * 32, smem, st>>>(a); break;
   }
   return check_launch();
 }

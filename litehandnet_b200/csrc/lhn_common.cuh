@@ -229,6 +229,34 @@ __device__ __forceinline__ float table_entry(const RenderGeom& g, int i, int W, 
   return !(arg > 0.0) ? exp_f32_from_f64(arg) : 0.f;
 }
 
+// Host: checks one scale of lhn_render_loss_multi / lhn_render_loss_backward_multi against the shared render
+// parameters and gives its feature stride (image_size / [W, H], or (image_size - 1) / ([W, H] - 1) for UDP, as
+// lhn_render_targets uses).
+inline int scale_geometry(const lhn_render_params* rp, int H, int W, float sigma, double& feat_x, double& feat_y) {
+  if (H <= 0 || W <= 0 || (int64_t)H * W > (1 << 30) || !(sigma > 0.f) || !(rp->image_w > 0.f) ||
+      !(rp->image_h > 0.f) || rp->loss_mode < LHN_LOSS_DISTANCE || rp->loss_mode > LHN_LOSS_JOINTS_MSE ||
+      rp->unbiased < 0 || rp->unbiased > 2)
+    return LHN_EINVAL;
+  if (rp->unbiased == 2) {
+    if (W < 2 || H < 2) return LHN_EINVAL;
+    feat_x = ((double)rp->image_w - 1.0) / (W - 1.0); feat_y = ((double)rp->image_h - 1.0) / (H - 1.0);
+  } else {
+    feat_x = (double)rp->image_w / W; feat_y = (double)rp->image_h / H;
+  }
+  return LHN_OK;
+}
+
+// Host: lets `kernel` take `smem` bytes of dynamic shared memory (above the 48 KB default only when asked for).
+inline int set_dynamic_smem(const void* kernel, size_t smem) {
+  if (smem <= 48 * 1024) return LHN_OK;
+  if (smem > 227 * 1024) return LHN_EINVAL;
+  if (cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) {
+    cudaGetLastError();
+    return LHN_EINVAL;
+  }
+  return LHN_OK;
+}
+
 // ---------------------------------------------------------------------------------------------
 // gradient stores and loss coefficients, shared by lhn_backward.cu and lhn_loss_grad.cu so that the
 // two-pass and the one-pass backward write bit-identical gradients

@@ -69,6 +69,28 @@ class _MultiHeatmapLossFn(torch.autograd.Function):
         return (None, None, None, None, None, *grads, *([None] * (2 * n)))
 
 
+class _FusedMultiHeatmapLossFn(torch.autograd.Function):
+    """SRHandNetLoss's scales with every target rendered in-kernel from the joints: ONE launch forward
+    (lhn_render_loss_multi), ONE launch backward (lhn_render_loss_backward_multi) for the outputs that need a
+    gradient."""
+
+    @staticmethod
+    def forward(ctx, render, reduction, loss_weights, joints, vis, *outputs):
+        outs = [o.detach() for o in outputs]
+        loss, sums, _, _ = ops.render_loss_multi(outs, joints, vis, render, loss_weights, reduction, want_weights=False)
+        ctx.save_for_backward(joints, vis, sums, *outs)
+        ctx.cfg = (render, reduction, loss_weights)
+        return loss[0]
+
+    @staticmethod
+    def backward(ctx, grad_out):
+        joints, vis, sums, *outs = ctx.saved_tensors
+        render, reduction, lw = ctx.cfg
+        grads = ops.render_loss_backward_multi(outs, joints, vis, render, sums, lw, reduction, grad_out,
+                                               needs=list(ctx.needs_input_grad[5:]))
+        return (None, None, None, None, None, *grads)
+
+
 class _FusedHeatmapLossFn(torch.autograd.Function):
     """The fused entry: target rendered in-kernel from the joints, one launch forward
     (lhn_fused_render_loss_decode without a refinement), lhn_render_loss_backward backward."""
@@ -361,7 +383,13 @@ class TopdownHeatmapLoss(nn.Module):
 class SRHandNetLoss(nn.Module):
     """loss/loss.py:7-66, heatmap-only branch (_forward_only_heatmap): sum_i loss_weight[i] *
     DistanceLoss(outputs[i], targets[i], w[i]) over the 4 scales.  The region-map branch
-    (pred_bbox with 24 channels) is out of scope (SURVEY §2 row 3/4)."""
+    (pred_bbox with 24 channels) is out of scope (SURVEY §2 row 3/4).
+
+    Fused entry (additive): when ``meta`` has no 'target' but has 'joints_3d' / 'joints_3d_visible', every scale's
+    target is rendered in-kernel — one launch forward, one backward — with SRHandNetGenerateTarget's settings:
+    cfg.DATASET.image_size, cfg.PIPELINE.sigma (one for every scale, or a list of one per scale; default
+    [2, 2, 2, 2]), cfg.PIPELINE.unbiased_encoding (default False) or UDP when cfg.PIPELINE.encoding == 'UDP'.  The
+    plane sizes are those of the outputs."""
 
     def __init__(self, cfg):
         super().__init__()
@@ -374,11 +402,51 @@ class SRHandNetLoss(nn.Module):
         self.num_out = 4
         self.loss_weight = cfg.LOSS.loss_weight
         assert len(self.loss_weight) == self.num_out
+        dataset = cfg.get('DATASET', None) or {}
+        pipeline = cfg.get('PIPELINE', None) or {}
+        self._image_size = dataset.get('image_size', None)
+        self._heatmap_size = dataset.get('heatmap_size', None)
+        self._sigma = pipeline.get('sigma', [2, 2, 2, 2])
+        self._unbiased = 'udp' if pipeline.get('encoding', 'MSRA') == 'UDP' else pipeline.get('unbiased_encoding', False)
 
     def forward(self, outputs, meta):
+        if 'target' not in meta and 'joints_3d' in meta and 'joints_3d_visible' in meta:
+            # the in-kernel render multiplies no per-joint weights into target_weight (generateTarget.py:156-157);
+            # every hand dataset forces them off (freihand_dataset.py:62) — refuse rather than silently ignore
+            ann = meta.get('ann_info', {}) if hasattr(meta, 'get') else {}
+            if meta.get('use_different_joint_weights', False) or (hasattr(ann, 'get') and ann.get('use_different_joint_weights', False)):
+                raise NotImplementedError("use_different_joint_weights: render the targets with SRHandNetGenerateTarget "
+                                          "and pass meta['target'] / meta['target_weight'] instead of the fused entry")
+            hs = self._heatmap_size
+            if isinstance(hs, (list, tuple)) and len(hs) and isinstance(hs[0], (list, tuple)):
+                got = [[int(outputs[i].shape[-1]), int(outputs[i].shape[-2])] for i in range(self.num_out)]
+                if [[int(x) for x in h] for h in hs] != got:
+                    raise ValueError(f"cfg.DATASET.heatmap_size {hs} does not match the outputs' [W, H] {got}")
+            if self._image_size is None:
+                raise ValueError("the fused SRHandNetLoss entry needs cfg.DATASET.image_size")
+            return self.forward_fused(outputs, meta['joints_3d'], meta['joints_3d_visible'], self._image_size,
+                                      self._sigma, self._unbiased)
         target = meta['target']
         target_weight = meta['target_weight']
         return self._forward_only_heatmap(outputs, target, target_weight)
+
+    def forward_fused(self, outputs, joints_3d, joints_3d_visible, image_size, sigmas=(2, 2, 2, 2),
+                      unbiased_encoding=False):
+        """The loss of ``forward`` with every scale's target rendered in-kernel from the joints (image_size [w, h];
+        sigmas: one for every scale or one per scale; unbiased_encoding False / True / 'udp').  Returns
+        (loss, dict(kpt_loss=float))."""
+        outs = [outputs[i] for i in range(self.num_out)]
+        for o in outs:
+            L.require_cuda(o, "output")
+        device = outs[-1].device
+        render = dict(loss_mode=self.mse_loss._mode, image_size=tuple(image_size),
+                      sigma=list(sigmas) if isinstance(sigmas, (list, tuple)) else sigmas,
+                      unbiased=unbiased_encoding, pos_value=self.mse_loss.value)
+        joints = _as_cuda(joints_3d, device)
+        vis = _as_cuda(joints_3d_visible, device)
+        loss = _FusedMultiHeatmapLossFn.apply(render, self.mse_loss.reduction, [float(x) for x in self.loss_weight],
+                                              joints, vis, *outs)
+        return loss, dict(kpt_loss=loss.item())
 
     def _forward_only_heatmap(self, outputs, targets, target_weight):
         device = outputs[-1].device

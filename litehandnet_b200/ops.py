@@ -429,6 +429,110 @@ def loss_mse_multi(outputs, targets, weights, loss_mode, pos_value=0.5, reductio
     return loss, sums, per
 
 
+def _loss_scales(outputs, joints, vis, render, loss_weights, what):
+    """Checks the per-scale inputs of the multi-scale rendered-target loss and builds its lhn_loss_scale array.
+    Returns (scales, keep-alive list, dtype code, B, K, render params, joints, vis)."""
+    n = len(outputs)
+    if n < 1 or n > L.LOSS_MAX_TENSORS:
+        raise L.LhnError(f"{what} takes 1..{L.LOSS_MAX_TENSORS} scales, got {n}")
+    joints = _f32c(joints, "joints")
+    vis = _f32c(vis, "vis")
+    if vis.dim() == 2:
+        vis = vis.unsqueeze(-1).contiguous()
+    sig = list(render["sigma"]) if isinstance(render["sigma"], (list, tuple)) else [render["sigma"]] * n
+    if len(sig) != n:
+        raise L.LhnError(f"{what}: {len(sig)} sigmas for {n} scales")
+    lw = [1.0] * n if loss_weights is None else [float(x) for x in loss_weights]
+    if len(lw) != n:
+        raise L.LhnError(f"{what}: {len(lw)} loss weights for {n} scales")
+    rp = _render_params(render["loss_mode"], render["image_size"], 1.0, render.get("unbiased", True),
+                        render.get("pos_value", 0.5))
+    scales = (L.LossScale * n)()
+    keep = []
+    B = K = None
+    for i, o in enumerate(outputs):
+        L.require_cuda(o, f"output {i}")
+        if o.device != joints.device:
+            raise L.LhnError(f"{what}: output {i} is on {o.device}, the joints on {joints.device}")
+        if o.dtype != outputs[0].dtype:
+            raise L.LhnError(f"{what}: all outputs must share one dtype ({outputs[0].dtype} and {o.dtype})")
+        if o.dim() != 4:
+            raise L.LhnError(f"{what}: output {i} must be [B,K,H,W], got {tuple(o.shape)}")
+        v, Bi, Ki, H, W, sb, sc = _plane_view(o.detach(), f"output {i}")
+        if B is None:
+            B, K = Bi, Ki
+        elif (Bi, Ki) != (B, K):
+            raise L.LhnError(f"{what}: output {i} is [{Bi},{Ki},..], output 0 [{B},{K},..]: B and K must agree")
+        keep.append(v)
+        s = scales[i]
+        s.output, s.stride_b, s.stride_c, s.H, s.W = v.data_ptr(), sb, sc, H, W
+        s.sigma, s.loss_weight = float(sig[i]), lw[i]
+    if joints.dim() != 3 or joints.shape[0] != B or joints.shape[1] != K or joints.shape[2] < 2:
+        raise L.LhnError(f"{what}: joints must be [B={B}, K={K}, >=2], got {tuple(joints.shape)}")
+    if vis.dim() != 3 or vis.shape[0] != B or vis.shape[1] != K:
+        raise L.LhnError(f"{what}: joints_visible must be [B={B}, K={K}(, >=1)], got {tuple(vis.shape)}")
+    return scales, keep, L.dtype_code(keep[0]), B, K, rp, joints, vis
+
+
+@_on_device
+def render_loss_multi(outputs, joints, vis, render, loss_weights=None, reduction="mean", want_weights=True):
+    """lhn_render_loss_multi: sum_i loss_weights[i] * DistanceLoss / JointsDistanceLoss of outputs[i] against the
+    target rendered in-kernel from the joints (SRHandNetLoss's scales, loss/loss.py:59-66), in ONE launch.
+    outputs: up to 8 [B,K,H_i,W_i] tensors of one dtype (channel-sliced views need no copy); joints [B,K,>=2],
+    vis [B,K(,>=1)]; render = dict(loss_mode, image_size, sigma (one for every scale, or a list of one per scale),
+    unbiased, pos_value).  Returns (loss f32[1], sums f64 [n,4], per_scale f32 [n], weights: a list of [B,K] f32
+    target_weight tensors, or None)."""
+    scales, keep, dt, B, K, rp, joints, vis = _loss_scales(outputs, joints, vis, render, loss_weights,
+                                                           "render_loss_multi")
+    n = len(outputs)
+    dev = keep[0].device
+    weights = None
+    if want_weights:
+        weights = [torch.empty((B, K), dtype=torch.float32, device=dev) for _ in range(n)]
+        for s, w in zip(scales, weights):
+            s.out_weight = w.data_ptr()
+    sums = torch.empty((n, 4), dtype=torch.float64, device=dev)
+    per = torch.empty(n, dtype=torch.float32, device=dev)
+    loss = torch.empty(1, dtype=torch.float32, device=dev)
+    ws = _loss_workspace(dev)
+    rc = L.lib().lhn_render_loss_multi(n, scales, dt, B, K, C.byref(rp), L.ptr(joints), joints.shape[2], L.ptr(vis),
+                                       vis.shape[2], int(reduction == "sum"), 1.0, L.ptr(ws), ws.numel(), L.ptr(sums),
+                                       L.ptr(per), L.ptr(loss), L.stream())
+    L.check(rc, "lhn_render_loss_multi")
+    return loss, sums, per, weights
+
+
+@_on_device
+def render_loss_backward_multi(outputs, joints, vis, render, sums, loss_weights=None, reduction="mean",
+                               grad_out=None, needs=None):
+    """lhn_render_loss_backward_multi: d loss / d outputs[i] for render_loss_multi's loss, every scale in ONE launch.
+    sums: the forward's f64 [n,4]; grad_out: the upstream gradient (CUDA tensor of one element, None = 1); needs: a
+    list of n booleans, the scales whose gradient is wanted (None = all).  Returns a list of contiguous gradients
+    like the outputs, None where not wanted."""
+    scales, keep, dt, B, K, rp, joints, vis = _loss_scales(outputs, joints, vis, render, loss_weights,
+                                                           "render_loss_backward_multi")
+    n = len(outputs)
+    sums = L.require_cuda(sums, "sums")
+    if sums.dtype != torch.float64 or sums.numel() != 4 * n or not sums.is_contiguous():
+        raise L.LhnError(f"sums must be a contiguous f64 [{n},4] tensor")
+    grads = []
+    for i, o in enumerate(outputs):
+        if needs is None or needs[i]:
+            g = torch.empty(o.shape, dtype=o.dtype, device=o.device)
+            scales[i].grad = g.data_ptr()
+            grads.append(g)
+        else:
+            grads.append(None)
+    if all(g is None for g in grads):
+        return grads
+    gkeep, gp = _grad_out_ptr(grad_out, keep[0].device)
+    rc = L.lib().lhn_render_loss_backward_multi(n, scales, dt, B, K, C.byref(rp), L.ptr(joints), joints.shape[2],
+                                                L.ptr(vis), vis.shape[2], L.ptr(sums), int(reduction == "sum"), gp,
+                                                L.stream())
+    L.check(rc, "lhn_render_loss_backward_multi")
+    return grads
+
+
 def _grad_out_ptr(grad_out, device):
     if grad_out is None:
         return None, None

@@ -449,12 +449,14 @@ LHN_API int lhn_loss_mse_multi(int n_tensors, const void* const* outputs, const 
  * LHN_LOSS_MAX_TENSORS descriptors. */
 typedef struct {
   const void* output;      /* [B, K, H, W] of `dtype`, planes contiguous, element strides stride_b / stride_c */
-  void* grad;              /* backward: contiguous [B, K, H, W] of `dtype`, or NULL to skip this scale; forward: unused */
-  float* out_weight;       /* forward: f32 [B*K] target_weight of this scale, or NULL; backward: unused */
+  void* grad;              /* backward, one pass: contiguous [B, K, H, W] of `dtype`, or NULL to skip this scale's
+                              gradient; forward: unused */
+  float* out_weight;       /* forward, one pass: f32 [B*K] target_weight of this scale, or NULL; backward: unused */
   int64_t stride_b, stride_c;
   int32_t H, W;
   float sigma;
-  float loss_weight;       /* forward: the weight of this scale's term; backward: its gradient's scale */
+  float loss_weight;       /* forward: the weight of this scale's term; backward: its gradient's scale; one pass:
+                              both */
 } lhn_loss_scale;
 
 /* Forward, ONE launch: the grid dealing, fixed-order two-level reduction and last-CTA finalise of
@@ -475,6 +477,34 @@ LHN_API int lhn_render_loss_backward_multi(int n_scales, const lhn_loss_scale* s
                                            const lhn_render_params* rp, const float* joints, int joints_stride,
                                            const float* vis, int vis_stride, const double* sums, int sum_reduction,
                                            const float* grad_out, lhn_stream_t stream);
+
+/* The loss AND every wanted scale's gradient in one pass over the outputs (one read, one write): the inputs of
+ * lhn_render_loss_multi, and it writes what that entry point writes — out_weight per scale, sums [n_scales, 4] with
+ * N_pos and numel bit for bit its values (S_pos, S_neg may differ in the last bits), per_scale_loss, loss.  Scale i's
+ * grad (NULL = not wanted; the scale is still read for its loss) receives d loss / d output for an upstream gradient
+ * grad_scale[0] (f32 [1] device pointer, NULL = 1), loss_weight_i being both the term's weight and the gradient's
+ * scale: bit for bit what lhn_render_loss_backward_multi writes from these sums with grad_out = grad_scale.  `scale`
+ * multiplies the reported loss only, as in lhn_render_loss_multi.  used_scale (f32 [1], optional) receives the
+ * upstream value assumed.  Two launches: the balanced loss's N_pos per scale is counted from the joints alone (skipped
+ * for the other modes and for pos_value >= 1), then one warp per plane streams every scale behind that count.
+ * workspace: lhn_render_loss_grad_multi_workspace_bytes(n_scales, B, K) bytes (0 for invalid arguments), 16-byte
+ * aligned, zero before the first call and left zero; bitwise reproducible for a given shape and device. */
+LHN_API int64_t lhn_render_loss_grad_multi_workspace_bytes(int n_scales, int64_t B, int K);
+LHN_API int lhn_render_loss_grad_multi(int n_scales, const lhn_loss_scale* scales, int dtype, int64_t B, int K,
+                                       const lhn_render_params* rp, const float* joints, int joints_stride,
+                                       const float* vis, int vis_stride, int sum_reduction, float scale,
+                                       void* workspace, int64_t workspace_bytes, double* sums, float* per_scale_loss,
+                                       float* loss, const float* grad_scale, float* used_scale, lhn_stream_t stream);
+/* The backward of lhn_render_loss_grad_multi: lhn_render_loss_backward_multi's arguments plus used_scale (required)
+ * and recomputed (int32 [1], optional).  If grad_out[0] (NULL = 1) is bitwise equal to used_scale[0], the gradients
+ * already in the scales' grad buffers are the answer and nothing is written (recomputed = 0); otherwise every wanted
+ * gradient is rewritten exactly as lhn_render_loss_backward_multi would (recomputed = 1).  With no gradient wanted it
+ * launches nothing. */
+LHN_API int lhn_render_loss_backward_multi_cond(int n_scales, const lhn_loss_scale* scales, int dtype, int64_t B,
+                                                int K, const lhn_render_params* rp, const float* joints,
+                                                int joints_stride, const float* vis, int vis_stride,
+                                                const double* sums, int sum_reduction, const float* grad_out,
+                                                const float* used_scale, int32_t* recomputed, lhn_stream_t stream);
 
 /* ---- SimDRLoss with its two nn.Linear heads fused (centernet_simdr_loss.py:42-69) -------------------------------
  * pred_x | pred_y = heatmap.flatten(2) @ [Wx ; Wy]^T + [bx ; by], then KLDiscretLoss (:27-39) — ONE tcgen05 kernel:

@@ -46,6 +46,7 @@ EXPORTS = [
     "lhn_vector_nms", "lhn_refine_points", "lhn_decode_heatmap_roi", "lhn_box_nms", "lhn_render_region_wh", "lhn_dark_refine_points",
     "lhn_k1_last_launch", "lhn_simdr_last_launch",
     "lhn_render_loss_multi_workspace_bytes", "lhn_render_loss_multi", "lhn_render_loss_backward_multi",
+    "lhn_render_loss_grad_multi_workspace_bytes", "lhn_render_loss_grad_multi", "lhn_render_loss_backward_multi_cond",
 ]
 
 
@@ -153,6 +154,13 @@ def _declare(lib):
                                           vp, i32, i32, f32, vp, i64, vp, vp, vp, vp]
     lib.lhn_render_loss_backward_multi.argtypes = [i32, C.POINTER(LossScale), i32, i64, i32, C.POINTER(RenderParams),
                                                    vp, i32, vp, i32, vp, i32, vp, vp]
+    lib.lhn_render_loss_grad_multi_workspace_bytes.argtypes = [i32, i64, i32]
+    lib.lhn_render_loss_grad_multi_workspace_bytes.restype = i64
+    lib.lhn_render_loss_grad_multi.argtypes = [i32, C.POINTER(LossScale), i32, i64, i32, C.POINTER(RenderParams), vp,
+                                               i32, vp, i32, i32, f32, vp, i64, vp, vp, vp, vp, vp, vp]
+    lib.lhn_render_loss_backward_multi_cond.argtypes = [i32, C.POINTER(LossScale), i32, i64, i32,
+                                                        C.POINTER(RenderParams), vp, i32, vp, i32, vp, i32, vp, vp, vp,
+                                                        vp]
     lib.lhn_loss_finalize.argtypes = [vp, i32, i32, f32, vp, i32, vp]
     lib.lhn_render_targets.argtypes = [vp, i32, vp, i32, i64, i32, i32, i32, C.POINTER(RenderParams),
                                        vp, vp, vp]

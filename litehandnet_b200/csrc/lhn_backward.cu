@@ -152,11 +152,20 @@ struct RenderBwdMultiArgs {
   int unbiased, loss_mode, sum_reduction, tab_stride;
   float pos_value;
   const double* sums; const float* grad_out;
+  const float* used_in; int* recomputed;      // COND only: the upstream value the one-pass forward assumed
 };
 
-template <typename T>
+// COND: the backward of lhn_render_loss_grad_multi — nothing to do when grad_out is bitwise the value the forward's
+// gradients assumed, else exactly the unconditional kernel's work (COND = false compiles to the code it had before)
+template <typename T, bool COND>
 __global__ void __launch_bounds__(kBwdMultiWarps * 32) render_loss_backward_multi_kernel(
     const __grid_constant__ RenderBwdMultiArgs a) {
+  if constexpr (COND) {
+    const float go = a.grad_out ? a.grad_out[0] : 1.f;
+    const bool same = __float_as_uint(go) == __float_as_uint(a.used_in[0]);
+    if (blockIdx.x == 0 && threadIdx.x == 0 && a.recomputed) a.recomputed[0] = same ? 0 : 1;
+    if (same) return;
+  }
   extern __shared__ float4 btab4[];
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int64_t gw = (int64_t)blockIdx.x * kBwdMultiWarps + warp;
@@ -311,11 +320,11 @@ extern "C" int lhn_render_loss_backward(const void* hm, int dtype, int64_t B, in
   return check_launch();
 }
 
-extern "C" int lhn_render_loss_backward_multi(int n_scales, const lhn_loss_scale* scales, int dtype, int64_t B,
-                                              int K, const lhn_render_params* rp, const float* joints,
-                                              int joints_stride, const float* vis, int vis_stride,
-                                              const double* sums, int sum_reduction, const float* grad_out,
-                                              lhn_stream_t stream) {
+// lhn_render_loss_backward_multi and, with used_scale != NULL, its conditional form
+static int backward_multi(int n_scales, const lhn_loss_scale* scales, int dtype, int64_t B, int K,
+                          const lhn_render_params* rp, const float* joints, int joints_stride, const float* vis,
+                          int vis_stride, const double* sums, int sum_reduction, const float* grad_out,
+                          const float* used_scale, int32_t* recomputed, lhn_stream_t stream) {
   if (n_scales < 1 || n_scales > LHN_LOSS_MAX_TENSORS || !scales || !rp || !joints || !vis || !sums || B <= 0 ||
       K <= 0 || joints_stride < 2 || vis_stride < 1)
     return LHN_EINVAL;
@@ -338,20 +347,39 @@ extern "C" int lhn_render_loss_backward_multi(int n_scales, const lhn_loss_scale
   a.joints = joints; a.joints_stride = joints_stride; a.vis = vis; a.vis_stride = vis_stride;
   a.unbiased = rp->unbiased; a.loss_mode = rp->loss_mode; a.sum_reduction = sum_reduction;
   a.tab_stride = (tab + 3) & ~3; a.pos_value = rp->pos_value; a.sums = sums; a.grad_out = grad_out;
+  a.used_in = used_scale; a.recomputed = recomputed;
   const int64_t blocks = (a.n * a.BK + kBwdMultiWarps - 1) / kBwdMultiWarps;
   if (blocks > 0x7fffffffLL) return LHN_EINVAL;
   const size_t smem = (size_t)kBwdMultiWarps * a.tab_stride * sizeof(float);
-  const void* fn = dtype == LHN_F32 ? (const void*)render_loss_backward_multi_kernel<float>
-                 : dtype == LHN_BF16 ? (const void*)render_loss_backward_multi_kernel<__nv_bfloat16>
-                                     : (const void*)render_loss_backward_multi_kernel<__half>;
-  if (set_dynamic_smem(fn, smem) != LHN_OK) return LHN_EINVAL;
-  cudaStream_t st = (cudaStream_t)stream;
-  switch (dtype) {
-    case LHN_F32: render_loss_backward_multi_kernel<float><<<(unsigned)blocks, kBwdMultiWarps * 32, smem, st>>>(a); break;
-    case LHN_BF16: render_loss_backward_multi_kernel<__nv_bfloat16><<<(unsigned)blocks, kBwdMultiWarps * 32, smem, st>>>(a); break;
-    default: render_loss_backward_multi_kernel<__half><<<(unsigned)blocks, kBwdMultiWarps * 32, smem, st>>>(a); break;
-  }
+  const bool cond = used_scale != nullptr;
+  void (*fn)(RenderBwdMultiArgs) =
+      dtype == LHN_F32 ? (cond ? render_loss_backward_multi_kernel<float, true> : render_loss_backward_multi_kernel<float, false>)
+    : dtype == LHN_BF16 ? (cond ? render_loss_backward_multi_kernel<__nv_bfloat16, true>
+                                : render_loss_backward_multi_kernel<__nv_bfloat16, false>)
+                        : (cond ? render_loss_backward_multi_kernel<__half, true> : render_loss_backward_multi_kernel<__half, false>);
+  if (set_dynamic_smem((const void*)fn, smem) != LHN_OK) return LHN_EINVAL;
+  fn<<<(unsigned)blocks, kBwdMultiWarps * 32, smem, (cudaStream_t)stream>>>(a);
   return check_launch();
+}
+
+extern "C" int lhn_render_loss_backward_multi(int n_scales, const lhn_loss_scale* scales, int dtype, int64_t B,
+                                              int K, const lhn_render_params* rp, const float* joints,
+                                              int joints_stride, const float* vis, int vis_stride,
+                                              const double* sums, int sum_reduction, const float* grad_out,
+                                              lhn_stream_t stream) {
+  return backward_multi(n_scales, scales, dtype, B, K, rp, joints, joints_stride, vis, vis_stride, sums,
+                        sum_reduction, grad_out, nullptr, nullptr, stream);
+}
+
+extern "C" int lhn_render_loss_backward_multi_cond(int n_scales, const lhn_loss_scale* scales, int dtype, int64_t B,
+                                                   int K, const lhn_render_params* rp, const float* joints,
+                                                   int joints_stride, const float* vis, int vis_stride,
+                                                   const double* sums, int sum_reduction, const float* grad_out,
+                                                   const float* used_scale, int32_t* recomputed,
+                                                   lhn_stream_t stream) {
+  if (!used_scale) return LHN_EINVAL;
+  return backward_multi(n_scales, scales, dtype, B, K, rp, joints, joints_stride, vis, vis_stride, sums,
+                        sum_reduction, grad_out, used_scale, recomputed, stream);
 }
 
 extern "C" int64_t lhn_simdr_backward_workspace_bytes(int K) { return K > 0 ? (int64_t)K * 4 : 0; }

@@ -298,6 +298,16 @@ __device__ __forceinline__ void loss_coefs(const double* sums, int loss_mode, in
   cpos = (float)(cp * g); cneg = (float)(cn * g);
 }
 
+// one loss from its f64 sums (S_pos, S_neg, N_pos, numel): the finalise of lhn_loss_mse_multi, lhn_render_loss_multi
+// and lhn_render_loss_grad_multi
+__device__ __forceinline__ double finalize_loss(double sp, double sn, double npos, double numel, int loss_mode, int sum_reduction) {
+  double v;
+  if (loss_mode == LHN_LOSS_DISTANCE_BALANCE) v = 0.1 * sp / (npos + 1.0) + sn / (numel - npos + 1.0);
+  else if (loss_mode == LHN_LOSS_JOINTS_MSE) v = 0.5 * (sp + sn) / numel;
+  else v = (sp + sn) / numel;
+  return sum_reduction ? v * numel : v;
+}
+
 // ---------------------------------------------------------------------------------------------
 // mbarrier + TMA bulk copy (cp.async.bulk, 1-D: no tensor map needed for contiguous planes)
 // ---------------------------------------------------------------------------------------------

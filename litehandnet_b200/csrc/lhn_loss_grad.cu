@@ -401,6 +401,291 @@ __global__ void __launch_bounds__(kGradThreads, 4) render_loss_backward_cond_ker
   }
 }
 
+// ==== SRHandNetLoss's scales: loss and gradient in one pass over the outputs (lhn_render_loss_grad_multi) ==========
+// Two launches.  The count kernel reads only the joints and adds each scale's N_pos (the forward's window, as above)
+// into a u64 counter per scale.  The stream kernel is lhn_render_loss_backward_multi's grid — one warp per plane,
+// warp-private tables, no grid barrier, so as many CTAs per SM as registers allow — launched with programmatic stream
+// serialization behind the count: a warp issues its plane's first loads and evaluates its tables, THEN waits for the
+// count (griddepcontrol.wait), forms the coefficients and writes the gradient while it accumulates the loss.  Scale
+// i owns CTAs [cta_begin_i, cta_begin_{i+1}), so a CTA's row belongs to one scale; the last CTA (ticket) adds the rows
+// per scale in a fixed order, finalises as lhn_render_loss_multi does and zeroes the counters, ticket and rows.
+constexpr int kGmWarps = 8;
+constexpr int kGmPrefetch = 4;          // chunks per lane whose loads go out before the wait on the count
+constexpr int kGmMaxScales = LHN_LOSS_MAX_TENSORS;
+constexpr int kGmWsRows = 256;          // workspace: [0, 64) N_pos per scale (u64), [64] ticket; rows from byte 256
+
+struct GradMultiScale {
+  const void* out; void* grad; float* w_out;
+  int64_t stride_b, stride_c;
+  double feat_x, feat_y;
+  float sigma, loss_weight, pos_radius;
+  int H, W, cta_begin;
+};
+
+struct GradMultiArgs {
+  GradMultiScale s[kGmMaxScales];
+  int n, K, cta_end;
+  int64_t BK;
+  const float* joints; int joints_stride;
+  const float* vis; int vis_stride;
+  int unbiased, loss_mode, sum_reduction, tab_stride, count, window;
+  float pos_value, scale;
+  const float* grad_scale; float* used_scale;
+  unsigned long long* npos; unsigned int* ticket; double* rows;
+  double* sums_out; float* per_scale; float* loss_out;
+};
+
+__device__ __forceinline__ void grid_dep_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
+__device__ __forceinline__ void grid_dep_launch() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
+
+__device__ __forceinline__ RenderGeom gm_geom(const GradMultiArgs& a, const GradMultiScale& s, int64_t p) {
+  return render_geom(a.joints[p * a.joints_stride], a.joints[p * a.joints_stride + 1], a.vis[p * a.vis_stride],
+                     (double)s.sigma, a.unbiased, s.feat_x, s.feat_y, 0, 0.0, 0.0, s.W, s.H);
+}
+
+// N_pos per scale from the joints.  window: 0 < value < 1, one thread per plane over the window around the joint
+// (render_loss_grad_kernel's loop); else (value <= 0) the whole plane, one warp per plane with its tables in shared
+// memory.  Integer sums: exact and independent of order.
+__global__ void __launch_bounds__(256) render_count_multi_kernel(const __grid_constant__ GradMultiArgs a) {
+  grid_dep_launch();                                      // the stream kernel may start its loads now
+  extern __shared__ float4 ctab4[];
+  __shared__ unsigned int cnt[kGmMaxScales];
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  if (tid < kGmMaxScales) cnt[tid] = 0u;
+  __syncthreads();
+  const int64_t total = a.n * a.BK;
+  if (a.window) {
+    const int64_t t = (int64_t)blockIdx.x * blockDim.x + tid;
+    if (t < total) {
+      const int i = (int)(t / a.BK);
+      const int64_t p = t - i * a.BK;
+      const GradMultiScale& s = a.s[i];
+      const RenderGeom g = gm_geom(a, s, p);
+      unsigned int c = 0;
+      if (g.on) {
+        const double sig = (double)s.sigma, inv2s2 = 1.0 / (2.0 * sig * sig);
+        const float rad = s.pos_radius;
+        const int W = s.W, H = s.H;
+        const int x_lo = max(0, (int)ceilf(g.cx - rad)), x_hi = min(W - 1, (int)floorf(g.cx + rad));
+        const int y_lo = max(0, (int)ceilf(g.cy - rad)), y_hi = min(H - 1, (int)floorf(g.cy + rad));
+        for (int yy = y_lo; yy <= y_hi; ++yy) {
+          const float gy = table_entry(g, W + yy, W, a.unbiased, inv2s2);
+          for (int xx = x_lo; xx <= x_hi; ++xx)
+            c += (table_entry(g, xx, W, a.unbiased, inv2s2) * gy > a.pos_value) ? 1u : 0u;
+        }
+      }
+      if (c) atomicAdd(&cnt[i], c);
+    }
+  } else {
+    const int64_t gw = (int64_t)blockIdx.x * (blockDim.x >> 5) + warp;
+    if (gw < total) {
+      const int i = (int)(gw / a.BK);
+      const int64_t p = gw - i * a.BK;
+      const GradMultiScale& s = a.s[i];
+      const int W = s.W, HW = s.W * s.H;
+      const RenderGeom g = gm_geom(a, s, p);
+      unsigned int c = 0;
+      if (g.on || a.pos_value < 0.f) {                    // off the image and value == 0: no element counts
+        float* wt = reinterpret_cast<float*>(ctab4) + warp * a.tab_stride;
+        const double sig = (double)s.sigma, inv2s2 = 1.0 / (2.0 * sig * sig);
+        for (int j = lane; j < W + s.H; j += 32) wt[j] = table_entry(g, j, W, a.unbiased, inv2s2);
+        __syncwarp();
+        for (int e = lane; e < HW; e += 32) {
+          const int ry = e / W, rx = e - ry * W;
+          c += (wt[rx] * wt[W + ry] > a.pos_value) ? 1u : 0u;
+        }
+      }
+      c = __reduce_add_sync(0xffffffffu, c);
+      if (lane == 0 && c) atomicAdd(&cnt[i], c);
+    }
+  }
+  __syncthreads();
+  if (tid < a.n && cnt[tid]) atomicAdd(a.npos + tid, (unsigned long long)cnt[tid]);
+}
+
+template <typename T, int VE>
+__device__ __forceinline__ void gm_load(uint4 (&raw)[kGmPrefetch], const T* src, int lane, int nch) {
+#pragma unroll
+  for (int u = 0; u < kGmPrefetch; ++u)
+    if (lane + 32 * u < nch) raw[u] = ld_chunk<T, VE>(src + (size_t)(lane + 32 * u) * VE);
+}
+
+// chunk c (elements c*VE ...) of a plane: gradient (render_grad_plane's arithmetic per element) and the f32 loss sums
+template <typename T, int VE>
+__device__ __forceinline__ void gm_chunk(const uint4& raw, int c, int W, const float* ex, const float* ey, T* dst,
+                                         float wp, float wn, bool bal, float pv, float& sp, float& sn) {
+  float v[VE], gx[VE], gy[VE], r[VE];
+  unpack_chunk<T, VE>(raw, v);
+  const int e0 = c * VE;
+  if (W % VE == 0) {                                      // the chunk lies in one row
+    const int row = e0 / W, col = e0 - row * W;
+    const float y = ey[row];
+#pragma unroll
+    for (int j = 0; j < VE; j += (VE >= 4 ? 4 : 1)) {
+      if constexpr (VE >= 4) {
+        const float4 x4 = *reinterpret_cast<const float4*>(ex + col + j);
+        gx[j] = x4.x; gx[j + 1] = x4.y; gx[j + 2] = x4.z; gx[j + 3] = x4.w;
+        gy[j] = gy[j + 1] = gy[j + 2] = gy[j + 3] = y;
+      } else {
+        gx[j] = ex[col + j]; gy[j] = y;
+      }
+    }
+  } else {                                                // rows are not whole chunks (W = 14): per element
+#pragma unroll
+    for (int j = 0; j < VE; ++j) {
+      const int e = e0 + j, yy = e / W;
+      gx[j] = ex[e - yy * W]; gy[j] = ey[yy];
+    }
+  }
+#pragma unroll
+  for (int j = 0; j < VE; ++j) {
+    const float g = gx[j] * gy[j];
+    const float d = fmaf(-gx[j], gy[j], v[j]);
+    const bool pos = bal && g > pv;
+    r[j] = (pos ? wp : wn) * d;
+    const float l = d * d;
+    sp += pos ? l : 0.f; sn += pos ? 0.f : l;
+  }
+  if (dst) st_chunk<T, VE>(dst + e0, r);
+}
+
+template <typename T, int VE>
+__device__ __forceinline__ void gm_plane(const uint4 (&raw)[kGmPrefetch], const T* src, T* dst, int lane, int HW, int W,
+                                         const float* ex, const float* ey, float wp, float wn, bool bal, float pv,
+                                         float& sp, float& sn) {
+  const int nch = HW / VE;
+#pragma unroll
+  for (int u = 0; u < kGmPrefetch; ++u)
+    if (lane + 32 * u < nch) gm_chunk<T, VE>(raw[u], lane + 32 * u, W, ex, ey, dst, wp, wn, bal, pv, sp, sn);
+#pragma unroll 4
+  for (int c = lane + 32 * kGmPrefetch; c < nch; c += 32)
+    gm_chunk<T, VE>(ld_chunk<T, VE>(src + (size_t)c * VE), c, W, ex, ey, dst, wp, wn, bal, pv, sp, sn);
+}
+
+template <typename T>
+__global__ void __launch_bounds__(kGmWarps * 32) render_loss_grad_multi_kernel(const __grid_constant__ GradMultiArgs a) {
+  extern __shared__ float4 gtab4[];
+  __shared__ double red[kGmWarps][2];
+  __shared__ double tloss[kGmMaxScales];
+  __shared__ unsigned int s_last;
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  int i = 0;
+#pragma unroll
+  for (int j = 1; j < kGmMaxScales; ++j)
+    if (j < a.n && (int)blockIdx.x >= a.s[j].cta_begin) i = j;
+  const GradMultiScale& s = a.s[i];
+  const int W = s.W, HW = s.W * s.H;
+  const int64_t p = (int64_t)((int)blockIdx.x - s.cta_begin) * kGmWarps + warp;
+  const bool has = p < a.BK;                              // warp-uniform
+  float* ex = reinterpret_cast<float*>(gtab4) + warp * a.tab_stride;
+  float* ey = ex + W;
+  const T* src = nullptr;
+  T* dst = nullptr;
+  int ve = 1;
+  float w = 0.f;
+  uint4 raw[kGmPrefetch];
+  if (blockIdx.x == 0 && tid == 0 && a.used_scale) a.used_scale[0] = a.grad_scale ? a.grad_scale[0] : 1.f;
+  if (has) {
+    // the plane's first loads go out first; the joint geometry and the tables overlap them and the count
+    const int64_t b = p / a.K;
+    const int k = (int)(p - b * a.K);
+    src = reinterpret_cast<const T*>(s.out) + b * s.stride_b + (int64_t)k * s.stride_c;
+    dst = s.grad ? reinterpret_cast<T*>(s.grad) + p * (int64_t)HW : nullptr;
+    const uintptr_t al = reinterpret_cast<uintptr_t>(src) | reinterpret_cast<uintptr_t>(dst);
+    ve = (sizeof(T) == 2 && HW % 8 == 0 && al % 16 == 0) ? 8 : (HW % 4 == 0 && al % (4 * sizeof(T)) == 0) ? 4 : 1;
+    if constexpr (sizeof(T) == 2) {
+      if (ve == 8) gm_load<T, 8>(raw, src, lane, HW / 8);
+      else if (ve == 4) gm_load<T, 4>(raw, src, lane, HW / 4);
+      else gm_load<T, 1>(raw, src, lane, HW);
+    } else {
+      if (ve == 4) gm_load<T, 4>(raw, src, lane, HW / 4);
+      else gm_load<T, 1>(raw, src, lane, HW);
+    }
+    const RenderGeom g = gm_geom(a, s, p);
+    w = g.w;
+    if (s.w_out && lane == 0) s.w_out[p] = w;
+    const double sig = (double)s.sigma, inv2s2 = 1.0 / (2.0 * sig * sig);
+    for (int e = lane; e < W + s.H; e += 32) ex[e] = table_entry(g, e, W, a.unbiased, inv2s2);
+    __syncwarp();
+  }
+  if (a.count) grid_dep_wait();                           // N_pos of every scale is complete and visible
+  double acc_sp = 0.0, acc_sn = 0.0;
+  if (has) {
+    double sums[4] = {0.0, 0.0, a.count ? (double)__ldcg(a.npos + i) : 0.0, (double)a.BK * (double)HW};
+    float cpos, cneg;
+    loss_coefs(sums, a.loss_mode, a.sum_reduction, s.loss_weight, a.grad_scale, cpos, cneg);
+    if (a.loss_mode == LHN_LOSS_JOINTS_MSE) w *= w;
+    const float wp = w * cpos, wn = w * cneg;
+    const bool bal = a.loss_mode == LHN_LOSS_DISTANCE_BALANCE;
+    float sp = 0.f, sn = 0.f;
+    if constexpr (sizeof(T) == 2) {
+      if (ve == 8) gm_plane<T, 8>(raw, src, dst, lane, HW, W, ex, ey, wp, wn, bal, a.pos_value, sp, sn);
+      else if (ve == 4) gm_plane<T, 4>(raw, src, dst, lane, HW, W, ex, ey, wp, wn, bal, a.pos_value, sp, sn);
+      else gm_plane<T, 1>(raw, src, dst, lane, HW, W, ex, ey, wp, wn, bal, a.pos_value, sp, sn);
+    } else {
+      if (ve == 4) gm_plane<T, 4>(raw, src, dst, lane, HW, W, ex, ey, wp, wn, bal, a.pos_value, sp, sn);
+      else gm_plane<T, 1>(raw, src, dst, lane, HW, W, ex, ey, wp, wn, bal, a.pos_value, sp, sn);
+    }
+    acc_sp = (double)sp * (double)w;                      // the forward's per-plane weighting (w^2 for JOINTS_MSE)
+    acc_sn = (double)sn * (double)w;
+  }
+  acc_sp = warp_sum(acc_sp); acc_sn = warp_sum(acc_sn);
+  if (lane == 0) { red[warp][0] = acc_sp; red[warp][1] = acc_sn; }
+  __syncthreads();
+  if (tid == 0) {
+    double r0 = 0.0, r1 = 0.0;
+    for (int j = 0; j < kGmWarps; ++j) { r0 += red[j][0]; r1 += red[j][1]; }
+    __stcg(reinterpret_cast<double2*>(a.rows) + blockIdx.x, make_double2(r0, r1));
+    __threadfence();
+    s_last = (atomicAdd(a.ticket, 1u) == gridDim.x - 1) ? 1u : 0u;
+  }
+  __syncthreads();
+  if (!s_last) return;
+  // ---- last CTA: a group of warps per scale adds that scale's rows (thread-strided, every load in flight at once,
+  // a fixed shuffle tree, then the group's warps in order) and zeroes them behind it
+  __threadfence();
+  int wpt = 1;
+  while (wpt * 2 * a.n <= kGmWarps) wpt *= 2;
+  const int groups = kGmWarps / wpt, grp = warp / wpt, sub = warp % wpt;
+  double2* rows = reinterpret_cast<double2*>(a.rows);
+  for (int i0 = 0; i0 < a.n; i0 += groups) {
+    const int si = i0 + grp;
+    double v0 = 0.0, v1 = 0.0;
+    if (si < a.n) {
+      const int c0 = a.s[si].cta_begin, c1 = si + 1 < a.n ? a.s[si + 1].cta_begin : a.cta_end;
+#pragma unroll 8
+      for (int c = c0 + sub * 32 + lane; c < c1; c += wpt * 32) {
+        const double2 x = __ldcg(rows + c);
+        v0 += x.x; v1 += x.y;
+        __stcg(rows + c, make_double2(0.0, 0.0));
+      }
+      v0 = warp_sum(v0); v1 = warp_sum(v1);
+    }
+    __syncthreads();                                      // red[] is free
+    if (lane == 0) { red[warp][0] = v0; red[warp][1] = v1; }
+    __syncthreads();
+    if (si < a.n && sub == 0 && lane == 0) {
+      double sp = 0.0, sn = 0.0;
+      for (int j = 0; j < wpt; ++j) { sp += red[warp + j][0]; sn += red[warp + j][1]; }
+      const double npos = a.count ? (double)__ldcg(a.npos + si) : 0.0;
+      const double numel = (double)a.BK * (double)(a.s[si].W * a.s[si].H);
+      if (a.sums_out) { double* o = a.sums_out + 4 * si; o[0] = sp; o[1] = sn; o[2] = npos; o[3] = numel; }
+      const double l = finalize_loss(sp, sn, npos, numel, a.loss_mode, a.sum_reduction);
+      if (a.per_scale) a.per_scale[si] = (float)l;
+      tloss[si] = (double)((float)l) * (double)a.s[si].loss_weight;
+    }
+  }
+  __syncthreads();
+  if (tid == 0) {
+    float total = 0.f;
+    for (int j = 0; j < a.n; ++j) total += (float)tloss[j];
+    total *= a.scale;
+    if (a.loss_out) a.loss_out[0] = total;
+    for (int j = 0; j < a.n; ++j) a.npos[j] = 0ull;
+    *a.ticket = 0u;
+  }
+}
+
 }  // namespace lhn
 
 using namespace lhn;
@@ -545,4 +830,82 @@ extern "C" int lhn_render_loss_backward_cond(const void* hm, int dtype, int64_t 
   if (a.n_planes == 0) return LHN_OK;
   a.sums = sums; a.grad_scale = grad_out; a.used_in = used_scale; a.recomputed = recomputed;
   return dispatch_grad(a, dtype, true, (cudaStream_t)stream);
+}
+
+extern "C" int64_t lhn_render_loss_grad_multi_workspace_bytes(int n_scales, int64_t B, int K) {
+  if (n_scales < 1 || n_scales > kGmMaxScales || B <= 0 || K <= 0) return 0;
+  return kGmWsRows + 16 * (int64_t)n_scales * ((B * K + kGmWarps - 1) / kGmWarps);
+}
+
+extern "C" int lhn_render_loss_grad_multi(int n_scales, const lhn_loss_scale* scales, int dtype, int64_t B, int K,
+                                          const lhn_render_params* rp, const float* joints, int joints_stride,
+                                          const float* vis, int vis_stride, int sum_reduction, float scale,
+                                          void* workspace, int64_t workspace_bytes, double* sums,
+                                          float* per_scale_loss, float* loss, const float* grad_scale,
+                                          float* used_scale, lhn_stream_t stream) {
+  if (n_scales < 1 || n_scales > kGmMaxScales || !scales || !rp || !joints || !vis || !workspace || B <= 0 ||
+      K <= 0 || joints_stride < 2 || vis_stride < 1)
+    return LHN_EINVAL;
+  if (dtype != LHN_F32 && dtype != LHN_BF16 && dtype != LHN_F16) return LHN_EDTYPE;
+  const int64_t ctas_per_scale = (B * K + kGmWarps - 1) / kGmWarps;
+  if (ctas_per_scale * n_scales > 0x7fffffffLL) return LHN_EINVAL;
+  if (workspace_bytes < lhn_render_loss_grad_multi_workspace_bytes(n_scales, B, K)) return LHN_EWORKSPACE;
+  if ((uintptr_t)workspace % 16 || (sums && (uintptr_t)sums % 8)) return LHN_EALIGN;
+  GradMultiArgs a{};
+  a.n = n_scales;
+  int tab = 0;
+  const float pv = rp->pos_value;
+  for (int i = 0; i < n_scales; ++i) {
+    const lhn_loss_scale& sc = scales[i];
+    GradMultiScale& s = a.s[i];
+    if (!sc.output || scale_geometry(rp, sc.H, sc.W, sc.sigma, s.feat_x, s.feat_y) != LHN_OK) return LHN_EINVAL;
+    s.out = sc.output; s.grad = sc.grad; s.w_out = sc.out_weight;
+    s.stride_b = sc.stride_b; s.stride_c = sc.stride_c; s.H = sc.H; s.W = sc.W;
+    s.sigma = sc.sigma; s.loss_weight = sc.loss_weight;
+    // the fused forward's window of the positives, as fill_grad_args: same expression, same bits
+    const double sg = (double)sc.sigma;
+    s.pos_radius = (pv > 0.f && pv < 1.f) ? (float)(sg * sqrt(-2.0 * log((double)pv)) * 1.001 + 0.01) : 0.f;
+    s.cta_begin = (int)(ctas_per_scale * i);
+    if (sc.H + sc.W > tab) tab = sc.H + sc.W;
+  }
+  a.cta_end = (int)(ctas_per_scale * n_scales);
+  a.K = K; a.BK = B * K;
+  a.joints = joints; a.joints_stride = joints_stride; a.vis = vis; a.vis_stride = vis_stride;
+  a.unbiased = rp->unbiased; a.loss_mode = rp->loss_mode; a.sum_reduction = sum_reduction;
+  a.tab_stride = (tab + 3) & ~3; a.pos_value = pv; a.scale = scale;
+  // N_pos is needed by the balanced loss only, and no element exceeds a value >= 1 (nor a NaN one)
+  a.count = a.loss_mode == LHN_LOSS_DISTANCE_BALANCE && pv < 1.f;
+  a.window = pv > 0.f && pv < 1.f;
+  a.grad_scale = grad_scale; a.used_scale = used_scale;
+  unsigned char* ws = static_cast<unsigned char*>(workspace);
+  a.npos = reinterpret_cast<unsigned long long*>(ws);
+  a.ticket = reinterpret_cast<unsigned int*>(ws + 64);
+  a.rows = reinterpret_cast<double*>(ws + kGmWsRows);
+  a.sums_out = sums; a.per_scale = per_scale_loss; a.loss_out = loss;
+  const size_t smem = (size_t)kGmWarps * a.tab_stride * sizeof(float);
+  void (*kern)(GradMultiArgs) = dtype == LHN_F32 ? render_loss_grad_multi_kernel<float>
+                              : dtype == LHN_BF16 ? render_loss_grad_multi_kernel<__nv_bfloat16>
+                                                  : render_loss_grad_multi_kernel<__half>;
+  if (set_dynamic_smem((const void*)kern, smem) != LHN_OK) return LHN_EINVAL;
+  cudaStream_t st = (cudaStream_t)stream;
+  if (a.count) {
+    const int64_t total = a.n * a.BK;
+    const int64_t blocks = a.window ? (total + 255) / 256 : (total + 7) / 8;
+    const size_t csmem = a.window ? 0 : smem;
+    if (blocks > 0x7fffffffLL) return LHN_EINVAL;
+    if (!a.window && set_dynamic_smem((const void*)render_count_multi_kernel, csmem) != LHN_OK) return LHN_EINVAL;
+    render_count_multi_kernel<<<(unsigned)blocks, 256, csmem, st>>>(a);
+    const int rc = check_launch();
+    if (rc != LHN_OK) return rc;
+  }
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = dim3((unsigned)a.cta_end); cfg.blockDim = dim3(kGmWarps * 32);
+  cfg.dynamicSmemBytes = smem; cfg.stream = st;
+  cudaLaunchAttribute at[1];
+  at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
+  at[0].val.programmaticStreamSerializationAllowed = 1;
+  cfg.attrs = at; cfg.numAttrs = a.count ? 1 : 0;       // without the count, the outputs' producer is the predecessor
+  cudaError_t e = cudaLaunchKernelEx(&cfg, kern, a);
+  if (e != cudaSuccess) { set_last_error(e); return LHN_ECUDA; }
+  return check_launch();
 }

@@ -56,14 +56,6 @@ struct LossMultiArgs {
   float* loss_out;           // [1]
 };
 
-__device__ __forceinline__ double finalize_loss(double sp, double sn, double npos, double numel, int loss_mode, int sum_reduction) {
-  double v;
-  if (loss_mode == LHN_LOSS_DISTANCE_BALANCE) v = 0.1 * sp / (npos + 1.0) + sn / (numel - npos + 1.0);
-  else if (loss_mode == LHN_LOSS_JOINTS_MSE) v = 0.5 * (sp + sn) / numel;
-  else v = (sp + sn) / numel;
-  return sum_reduction ? v * numel : v;
-}
-
 // RENDER: plane loads issued per lane before the plane's tables are evaluated (a first round of the stream)
 constexpr int kRenderPrefetch = 4;
 

@@ -91,6 +91,36 @@ class _FusedMultiHeatmapLossFn(torch.autograd.Function):
         return (None, None, None, None, None, *grads)
 
 
+class _FusedMultiHeatmapLossOnePassFn(torch.autograd.Function):
+    """SRHandNetLoss's scales with the gradients written in the forward (lhn_render_loss_grad_multi: one read of the
+    outputs, one write of the gradients of those that need one).  The gradients assume the upstream value
+    ``expected``; the backward (lhn_render_loss_backward_multi_cond) returns them as they are when autograd delivers
+    exactly that value, and rewrites them as the two-launch backward would otherwise.  The gradient buffers are
+    allocated here, in the forward."""
+
+    @staticmethod
+    def forward(ctx, render, reduction, loss_weights, expected, joints, vis, *outputs):
+        outs = [o.detach() for o in outputs]
+        loss, sums, _, grads, used, _ = ops.render_loss_grad_multi(outs, joints, vis, render, loss_weights, reduction,
+                                                                   expected, needs=list(ctx.needs_input_grad[6:]),
+                                                                   want_weights=False)
+        ctx.save_for_backward(joints, vis, sums, used, *outs)
+        # the gradients are intermediates, kept on ctx and released in backward: handed back with no other reference,
+        # autograd adopts them as the outputs' .grad instead of copying them
+        ctx.grads = grads
+        ctx.cfg = (render, reduction, loss_weights)
+        return loss[0]
+
+    @staticmethod
+    def backward(ctx, grad_out):
+        joints, vis, sums, used, *outs = ctx.saved_tensors
+        grads, ctx.grads = ctx.grads, None
+        render, reduction, lw = ctx.cfg
+        ops.render_loss_backward_multi_cond(outs, joints, vis, render, sums, grads, used, lw, reduction, grad_out,
+                                            recomputed=_ONE_PASS_PROBE.get("recomputed"))
+        return (None, None, None, None, None, None, *grads)
+
+
 class _FusedHeatmapLossFn(torch.autograd.Function):
     """The fused entry: target rendered in-kernel from the joints, one launch forward
     (lhn_fused_render_loss_decode without a refinement), lhn_render_loss_backward backward."""
@@ -389,7 +419,8 @@ class SRHandNetLoss(nn.Module):
     target is rendered in-kernel — one launch forward, one backward — with SRHandNetGenerateTarget's settings:
     cfg.DATASET.image_size, cfg.PIPELINE.sigma (one for every scale, or a list of one per scale; default
     [2, 2, 2, 2]), cfg.PIPELINE.unbiased_encoding (default False) or UDP when cfg.PIPELINE.encoding == 'UDP'.  The
-    plane sizes are those of the outputs."""
+    plane sizes are those of the outputs.  cfg.LOSS.one_pass_grad = True (default False) computes the loss and the
+    gradients in one pass over the outputs when a gradient is needed (SRHandNetLoss.forward_fused(one_pass=True))."""
 
     def __init__(self, cfg):
         super().__init__()
@@ -408,6 +439,8 @@ class SRHandNetLoss(nn.Module):
         self._heatmap_size = dataset.get('heatmap_size', None)
         self._sigma = pipeline.get('sigma', [2, 2, 2, 2])
         self._unbiased = 'udp' if pipeline.get('encoding', 'MSRA') == 'UDP' else pipeline.get('unbiased_encoding', False)
+        # fused entry: loss and gradients in one pass over the outputs (forward_fused(one_pass=True))
+        self.one_pass_grad = bool(cfg.LOSS.get('one_pass_grad', False))
 
     def forward(self, outputs, meta):
         if 'target' not in meta and 'joints_3d' in meta and 'joints_3d_visible' in meta:
@@ -424,17 +457,25 @@ class SRHandNetLoss(nn.Module):
                     raise ValueError(f"cfg.DATASET.heatmap_size {hs} does not match the outputs' [W, H] {got}")
             if self._image_size is None:
                 raise ValueError("the fused SRHandNetLoss entry needs cfg.DATASET.image_size")
+            # the loss weights are applied inside the kernel: autograd delivers 1 to this loss
             return self.forward_fused(outputs, meta['joints_3d'], meta['joints_3d_visible'], self._image_size,
-                                      self._sigma, self._unbiased)
+                                      self._sigma, self._unbiased, one_pass=self.one_pass_grad)
         target = meta['target']
         target_weight = meta['target_weight']
         return self._forward_only_heatmap(outputs, target, target_weight)
 
     def forward_fused(self, outputs, joints_3d, joints_3d_visible, image_size, sigmas=(2, 2, 2, 2),
-                      unbiased_encoding=False):
+                      unbiased_encoding=False, one_pass=False, expected_grad_out=1.0):
         """The loss of ``forward`` with every scale's target rendered in-kernel from the joints (image_size [w, h];
         sigmas: one for every scale or one per scale; unbiased_encoding False / True / 'udp').  Returns
-        (loss, dict(kpt_loss=float))."""
+        (loss, dict(kpt_loss=float)).
+
+        one_pass=True (when grad is enabled and an output requires a gradient): the loss and d loss / d outputs come
+        from ONE pass over the outputs, and ``loss.backward()`` returns those gradients without reading the outputs
+        again — provided the upstream gradient of the loss is bitwise ``expected_grad_out`` (a float, or a 0-dim CUDA
+        tensor such as a gradient scaler's scale).  Any other upstream value is still correct: the backward then
+        recomputes the gradients as the default route does.  The gradient buffers are allocated in the forward rather
+        than in the backward."""
         outs = [outputs[i] for i in range(self.num_out)]
         for o in outs:
             L.require_cuda(o, "output")
@@ -444,8 +485,12 @@ class SRHandNetLoss(nn.Module):
                       unbiased=unbiased_encoding, pos_value=self.mse_loss.value)
         joints = _as_cuda(joints_3d, device)
         vis = _as_cuda(joints_3d_visible, device)
-        loss = _FusedMultiHeatmapLossFn.apply(render, self.mse_loss.reduction, [float(x) for x in self.loss_weight],
-                                              joints, vis, *outs)
+        lw = [float(x) for x in self.loss_weight]
+        if one_pass and torch.is_grad_enabled() and any(o.requires_grad for o in outs):
+            loss = _FusedMultiHeatmapLossOnePassFn.apply(render, self.mse_loss.reduction, lw, expected_grad_out,
+                                                         joints, vis, *outs)
+        else:
+            loss = _FusedMultiHeatmapLossFn.apply(render, self.mse_loss.reduction, lw, joints, vis, *outs)
         return loss, dict(kpt_loss=loss.item())
 
     def _forward_only_heatmap(self, outputs, targets, target_weight):

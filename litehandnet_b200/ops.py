@@ -533,6 +533,91 @@ def render_loss_backward_multi(outputs, joints, vis, render, sums, loss_weights=
     return grads
 
 
+_GRAD_MULTI_WS = {}
+
+
+def render_loss_grad_multi_workspace(device, n, B, K):
+    """Zeroed once per (device, stream), grown when a larger shape comes; lhn_render_loss_grad_multi leaves it zeroed."""
+    need = int(L.lib().lhn_render_loss_grad_multi_workspace_bytes(int(n), int(B), int(K)))
+    key = (str(device), torch.cuda.current_stream(device).cuda_stream)
+    ws = _GRAD_MULTI_WS.get(key)
+    if ws is None or ws.numel() < need:
+        ws = _GRAD_MULTI_WS[key] = torch.zeros(need, dtype=torch.uint8, device=device)
+    return ws
+
+
+@_on_device
+def render_loss_grad_multi(outputs, joints, vis, render, loss_weights=None, reduction="mean", grad_scale=None,
+                           needs=None, want_weights=True, workspace=None):
+    """render_loss_multi's loss and render_loss_backward_multi's gradients in ONE pass over the outputs
+    (lhn_render_loss_grad_multi).  The gradients are those of an upstream gradient ``grad_scale`` (float or one-element
+    CUDA tensor; None = 1); needs: a list of n booleans, the scales whose gradient is wanted (None = all; the others are
+    still read for the loss).  Returns (loss f32[1], sums f64 [n,4], per_scale f32 [n], gradients: a list of
+    contiguous tensors like the outputs, None where not wanted, used_scale f32[1], weights: a list of [B,K] f32
+    target_weight tensors, or None)."""
+    scales, keep, dt, B, K, rp, joints, vis = _loss_scales(outputs, joints, vis, render, loss_weights,
+                                                           "render_loss_grad_multi")
+    n = len(outputs)
+    dev = keep[0].device
+    grads = []
+    for i, o in enumerate(outputs):
+        if needs is None or needs[i]:
+            g = torch.empty(o.shape, dtype=o.dtype, device=dev)
+            scales[i].grad = g.data_ptr()
+            grads.append(g)
+        else:
+            grads.append(None)
+    weights = None
+    if want_weights:
+        weights = [torch.empty((B, K), dtype=torch.float32, device=dev) for _ in range(n)]
+        for s, w in zip(scales, weights):
+            s.out_weight = w.data_ptr()
+    sums = torch.empty((n, 4), dtype=torch.float64, device=dev)
+    per = torch.empty(n, dtype=torch.float32, device=dev)
+    loss = torch.empty(1, dtype=torch.float32, device=dev)
+    used = torch.empty(1, dtype=torch.float32, device=dev)
+    gkeep, gp = (None, None) if grad_scale is None else _scale_tensor(grad_scale, dev)
+    ws = workspace if workspace is not None else render_loss_grad_multi_workspace(dev, n, B, K)
+    rc = L.lib().lhn_render_loss_grad_multi(n, scales, dt, B, K, C.byref(rp), L.ptr(joints), joints.shape[2],
+                                            L.ptr(vis), vis.shape[2], int(reduction == "sum"), 1.0, L.ptr(ws),
+                                            ws.numel(), L.ptr(sums), L.ptr(per), L.ptr(loss), gp, L.ptr(used),
+                                            L.stream())
+    L.check(rc, "lhn_render_loss_grad_multi")
+    return loss, sums, per, grads, used, weights
+
+
+@_on_device
+def render_loss_backward_multi_cond(outputs, joints, vis, render, sums, grads, used_scale, loss_weights=None,
+                                    reduction="mean", grad_out=None, recomputed=None):
+    """Backward of render_loss_grad_multi (lhn_render_loss_backward_multi_cond): ``grads`` (its list, None where not
+    wanted) are left as they are when grad_out (None = 1) is bitwise the ``used_scale`` the forward assumed, else
+    overwritten as render_loss_backward_multi would write them.  recomputed: optional int32 [1] CUDA tensor, set to 0
+    or 1.  Returns grads."""
+    scales, keep, dt, B, K, rp, joints, vis = _loss_scales(outputs, joints, vis, render, loss_weights,
+                                                           "render_loss_backward_multi_cond")
+    n = len(outputs)
+    sums = L.require_cuda(sums, "sums")
+    if sums.dtype != torch.float64 or sums.numel() != 4 * n or not sums.is_contiguous():
+        raise L.LhnError(f"sums must be a contiguous f64 [{n},4] tensor")
+    if len(grads) != n:
+        raise L.LhnError(f"{len(grads)} gradients for {n} scales")
+    for i, (o, g) in enumerate(zip(outputs, grads)):
+        if g is None:
+            continue
+        if g.shape != o.shape or g.dtype != o.dtype or not g.is_contiguous() or g.device != o.device:
+            raise L.LhnError(f"gradient {i} must be a contiguous tensor of output {i}'s shape, dtype and device")
+        scales[i].grad = g.data_ptr()
+    if recomputed is not None and (recomputed.dtype != torch.int32 or recomputed.numel() != 1):
+        raise L.LhnError("recomputed must be an int32 tensor of one element")
+    gkeep, gp = _grad_out_ptr(grad_out, keep[0].device)
+    rc = L.lib().lhn_render_loss_backward_multi_cond(n, scales, dt, B, K, C.byref(rp), L.ptr(joints),
+                                                     joints.shape[2], L.ptr(vis), vis.shape[2], L.ptr(sums),
+                                                     int(reduction == "sum"), gp, L.ptr(used_scale),
+                                                     L.ptr(recomputed), L.stream())
+    L.check(rc, "lhn_render_loss_backward_multi_cond")
+    return grads
+
+
 def _grad_out_ptr(grad_out, device):
     if grad_out is None:
         return None, None

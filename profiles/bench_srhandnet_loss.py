@@ -1,13 +1,16 @@
-"""SRHandNetLoss forward + backward for one training step, three routes, on one GPU:
+"""SRHandNetLoss forward + backward for one training step, four routes, on one GPU:
   (a) today's route with the targets rendered on the GPU (render_srhandnet_targets, pred_bbox=False: one
       lhn_render_targets per scale), then lhn_loss_mse_multi and one lhn_loss_backward per scale;
   (b) today's route with the targets already resident (the dataloader case): lhn_loss_mse_multi + 4 backward launches;
-  (c) the fused route: lhn_render_loss_multi + lhn_render_loss_backward_multi.
-Reports CUDA-graph replay and eager medians per step, the two new kernels' times and their share of the copy peak
-(bytes from shapes: the forward reads the outputs, the backward reads them and writes the gradients), launches per step,
-and a parity check of (a) against (c).  Inputs rotate over more than the 126 MB L2 (the line says how many sets).
+  (c) the fused route: lhn_render_loss_multi + lhn_render_loss_backward_multi;
+  (d) the fused route in one pass (cfg.LOSS.one_pass_grad): lhn_render_loss_grad_multi (count + stream launch) +
+      lhn_render_loss_backward_multi_cond (a no-op for loss.backward()).
+Reports CUDA-graph replay and eager medians per step, the fused kernels' times and their share of the copy peak
+(bytes from shapes: the forward reads the outputs, the backward and the one-pass call read them and write the
+gradients), launches per step, and parity checks of (a) against (c) and of (d) against (c) (loss relative difference,
+gradients bit for bit).  Inputs rotate over more than the 126 MB L2 (the line says how many sets).
 
-    python profiles/bench_srhandnet_loss.py [--out profiles/r04_srhandnet_loss.txt]
+    python profiles/bench_srhandnet_loss.py [--out profiles/r05_srhandnet_one_pass.txt]
 """
 import argparse
 import math
@@ -74,6 +77,8 @@ def step_fn(route, sizes):
             loss = explicit(s["outs"], tg, tw)
         elif route == "b":
             loss = explicit(s["outs"], s["tg"], s["tw"])
+        elif route == "d":
+            loss = LS._FusedMultiHeatmapLossOnePassFn.apply(render_dict(), "mean", LW, 1.0, s["j"], s["v"], *s["outs"])
         else:
             loss = LS._FusedMultiHeatmapLossFn.apply(render_dict(), "mean", LW, s["j"], s["v"], *s["outs"])
         loss.backward()
@@ -152,7 +157,15 @@ def time_kernels(sets, reps):
                                               "mean", want_weights=False))
     tb = loop(lambda i: ops.render_loss_backward_multi([o.detach() for o in sets[i]["outs"]], sets[i]["j"],
                                                        sets[i]["v"], rd, fw[i][1], LW, "mean"))
-    return tf, tb
+    tg = loop(lambda i: ops.render_loss_grad_multi([o.detach() for o in sets[i]["outs"]], sets[i]["j"], sets[i]["v"],
+                                                   rd, LW, "mean", want_weights=False))
+    op = [ops.render_loss_grad_multi([o.detach() for o in s["outs"]], s["j"], s["v"], rd, LW, "mean", want_weights=False)
+          for s in sets]
+    one = torch.ones(1, device="cuda")
+    tcnd = loop(lambda i: ops.render_loss_backward_multi_cond([o.detach() for o in sets[i]["outs"]], sets[i]["j"],
+                                                              sets[i]["v"], rd, op[i][1], op[i][3], op[i][4], LW,
+                                                              "mean", one))
+    return tf, tb, tg, tcnd
 
 
 def launches(fn, s):
@@ -166,14 +179,40 @@ def launches(fn, s):
                "memcpy" not in e.name.lower() and "memset" not in e.name.lower())
 
 
+def one_pass_kernels(sizes, sets, reps=20):
+    """Device time of each kernel of route (d), from torch.profiler over `reps` steps in a run of their own: the count,
+    the stream and the conditional backward (mean per step, us)."""
+    from torch.profiler import ProfilerActivity, profile
+    fn = step_fn("d", sizes)
+    fn(sets[0])
+    torch.cuda.synchronize()
+    with profile(activities=[ProfilerActivity.CUDA]) as prof:
+        for r in range(reps):
+            fn(sets[r % len(sets)])
+        torch.cuda.synchronize()
+    t = {"count": 0.0, "stream": 0.0, "cond": 0.0}
+    for e in prof.events():
+        if e.device_type != torch.autograd.DeviceType.CUDA:
+            continue
+        key = ("count" if "render_count_multi_kernel" in e.name else "stream" if "render_loss_grad_multi_kernel" in e.name
+               else "cond" if "render_loss_backward_multi_kernel" in e.name else None)
+        if key:
+            t[key] += e.time_range.elapsed_us()
+    return {k: v / reps for k, v in t.items()}
+
+
 def parity(sizes, s):
-    fa, fc = step_fn("a", sizes), step_fn("c", sizes)
+    fa, fc, fd = step_fn("a", sizes), step_fn("c", sizes), step_fn("d", sizes)
     la = fa(s).item()
     ga = [o.grad.clone() for o in s["outs"]]
     lc = fc(s).item()
     gc = [o.grad.clone() for o in s["outs"]]
+    ld = fd(s).item()
+    gd = [o.grad.clone() for o in s["outs"]]
     dg = max(((x.float() - y.float()).abs().max() / y.float().abs().max().clamp_min(1e-30)).item() for x, y in zip(gc, ga))
-    return abs(lc - la) / abs(la), dg
+    same = sum(int(torch.equal(x.view(torch.int16 if x.element_size() == 2 else torch.int32),
+                               y.view(torch.int16 if y.element_size() == 2 else torch.int32))) for x, y in zip(gd, gc))
+    return abs(lc - la) / abs(la), dg, abs(ld - lc) / abs(lc), same
 
 
 def main():
@@ -193,20 +232,29 @@ def main():
                 row = f"sizes={sizes} B={B} {dtype}: outputs {nbytes / 1e6:.1f} MB x {nsets} sets " \
                       f"({nbytes * nsets / 2**20:.0f} MiB rotated)"
                 lines.append(row)
-                for route, label in (("a", "(a) render + explicit"), ("b", "(b) resident targets"), ("c", "(c) fused")):
+                for route, label in (("a", "(a) render + explicit"), ("b", "(b) resident targets"), ("c", "(c) fused"),
+                                     ("d", "(d) fused, one pass")):
                     fn = step_fn(route, sizes)
                     te = time_eager(fn, sets, args.reps)
                     tgph = time_graph(fn, sets, args.reps)
                     nl = launches(fn, sets[0])
                     lines.append(f"  {label:24s} eager {te:9.1f} us  graph {tgph:9.1f} us  launches/step {nl}")
-                tf, tb = time_kernels(sets, args.reps)
+                tf, tb, tg, tcnd = time_kernels(sets, args.reps)
                 lines.append(f"  lhn_render_loss_multi          {tf:9.1f} us  {nbytes / tf / 1e3:7.1f} GB/s  "
                              f"{100 * nbytes / (tf * 1e-6) / COPY_PEAK:5.1f} % of copy peak")
                 lines.append(f"  lhn_render_loss_backward_multi {tb:9.1f} us  {2 * nbytes / tb / 1e3:7.1f} GB/s  "
                              f"{100 * 2 * nbytes / (tb * 1e-6) / COPY_PEAK:5.1f} % of copy peak")
-                dl, dg = parity(sizes, sets[0])
+                lines.append(f"  lhn_render_loss_grad_multi     {tg:9.1f} us  {2 * nbytes / tg / 1e3:7.1f} GB/s  "
+                             f"{100 * 2 * nbytes / (tg * 1e-6) / COPY_PEAK:5.1f} % of copy peak  (count + stream launch)")
+                lines.append(f"  lhn_render_loss_backward_multi_cond, upstream as assumed {tcnd:9.1f} us (host-bound loop)")
+                kt = one_pass_kernels(sizes, sets)
+                lines.append(f"  (d) kernels, profiler: count {kt['count']:6.1f} us, stream {kt['stream']:6.1f} us "
+                             f"({100 * 2 * nbytes / (kt['stream'] * 1e-6) / COPY_PEAK:5.1f} % of copy peak), "
+                             f"conditional backward {kt['cond']:5.1f} us")
+                dl, dg, dd, same = parity(sizes, sets[0])
                 lines.append(f"  parity (a) vs (c): loss rel {dl:.2e}, gradient max |diff| / max |grad| {dg:.2e}")
-                print("\n".join(lines[-7:]), flush=True)
+                lines.append(f"  parity (d) vs (c): loss rel {dd:.2e}, gradients bit-equal {same} / {len(sizes)}")
+                print("\n".join(lines[-12:]), flush=True)
                 del sets
                 torch.cuda.empty_cache()
     os.makedirs(os.path.dirname(os.path.abspath(args.out)), exist_ok=True)
